@@ -2,6 +2,7 @@
 """Benchmark of the area-average interpolation hot path (BASELINE.json metric: output Mpixels/s, device-timed).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config 4] [--impl ours|reference] [--no-extra]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over the whole workload (default: BASELINE config 4, the 16384x16384
 float32 slice, 0.37x, 17.3 deg -> 7591x7591 canvas).  With N > 1 (torchrun, one process per GPU) the canvas is
@@ -43,6 +44,7 @@ sys.path.insert(0, ROOT)
 
 METRIC = "output Mpixels/s (device-timed)"
 UNIT = "Mpix/s"
+DUMP_BYTES = 32 << 20  # --dump-outputs: canvas sample size limit
 
 # BASELINE.json configs (SURVEY.md §8d fixes isocentres and generators); index = config number
 CONFIGS = {
@@ -320,8 +322,9 @@ class Bench:
 
     # -- one workload ----------------------------------------------------------------------------------------------------
     def measure(self, cfg_id, arith_name="auto", mode=1, steps=None, with_e2e=True, with_verify=True,
-                with_clocks=True, tag=None):
-        """Device-timed value, end-to-end value, roofline and verification of one BASELINE shape."""
+                with_clocks=True, tag=None, dump_dir=None):
+        """Device-timed value, end-to-end value, roofline and verification of one BASELINE shape; with `dump_dir`, the
+        canvas of the last timed step is written there (dump_canvas)."""
         torch, aai, args = self.torch, self.aai, self.args
         from area_average_interpolation_b200.sharding import band_for_rank, batch_slice
         from area_average_interpolation_b200.synthetic import synthetic_image_torch
@@ -409,6 +412,8 @@ class Bench:
         ms_step = self.max_over_ranks(e0.elapsed_time(e1)) / steps
         value = total_pixels / (ms_step * 1e-3) / 1e6
         band_ms = self.gather(e0.elapsed_time(e1) / steps)
+        if dump_dir:
+            self.dump_canvas(dump_dir, cfg, plan, dev_dst, band.row0 if band is not None else lo * plan.dst_h)
 
         # ---- end-to-end region (host buffers through the C ABI) --------------------------------------------------
         e2e = None
@@ -558,6 +563,24 @@ class Bench:
         torch.cuda.empty_cache()
         return res
 
+    def dump_canvas(self, out_dir, cfg, plan, dev_dst, first_row):
+        """Writes `out_dir`/canvas.npy: the canvas rows this workload's timed path produced, as float32 (float64 for a
+        float64 canvas), rows ordered over the whole workload (row r of slice k is row k * dst_h + r).  A canvas larger
+        than DUMP_BYTES is sampled: a fixed, seeded choice of rows in ascending order, the same for any number of GPUs.
+        `dev_dst` holds this rank's rows, starting at workload row `first_row`."""
+        torch = self.torch
+        local = dev_dst.flatten(0, 1) if cfg["batch"] > 1 else dev_dst
+        out_np = np.float64 if dev_dst.dtype == torch.float64 else np.float32
+        total = cfg["batch"] * plan.dst_h
+        n = min(total, DUMP_BYTES // (plan.dst_w * cfg["ch"] * np.dtype(out_np).itemsize))
+        rows = np.arange(total) if n == total else np.sort(np.random.default_rng(0).choice(total, n, replace=False))
+        mine = rows[(rows >= first_row) & (rows < first_row + local.shape[0])] - first_row
+        part = local[torch.as_tensor(mine, device=self.dev)].cpu().numpy().astype(out_np)
+        parts = self.gather(part)  # ranks hold consecutive row ranges in rank order
+        if self.rank == 0:
+            os.makedirs(out_dir, exist_ok=True)
+            np.save(os.path.join(out_dir, "canvas.npy"), np.concatenate(parts, axis=0))
+
     def _verify(self, cfg, cfg_id, plan, mode, arith, band, dev_dst, host_dst, step, seed, first_image):
         """(a) the end-to-end canvas equals, bit for bit, the canvas computed from the HBM-generated source (the upload /
         NVLink exchange delivered exactly the right bytes to the right rows); (b) first, middle and last row of this rank's
@@ -634,7 +657,8 @@ class Bench:
 def our_arm(args, cfg_id):
     b = Bench(args)
     cfg = CONFIGS[cfg_id]
-    head = b.measure(cfg_id, arith_name=args.arith, mode=args.mode, with_e2e=True, with_verify=not args.no_verify)
+    head = b.measure(cfg_id, arith_name=args.arith, mode=args.mode, with_e2e=True, with_verify=not args.no_verify,
+                     dump_dir=args.dump_outputs)
     plan, info = head.pop("_plan"), head.pop("_info")
     line = {
         "metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": b.world, "steps": args.steps,
@@ -691,7 +715,8 @@ def our_arm(args, cfg_id):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the headline workload (the `configs` records take min(K, 10), at least 3)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--config", type=int, default=4, choices=sorted(CONFIGS))
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
@@ -704,7 +729,16 @@ def main():
     ap.add_argument("--peer-chunks", type=int, default=0, help="N>1: upload chunks per owner rank of the peer group (1..8)")
     ap.add_argument("--no-peer", action="store_true",
                     help="N>1: every rank uploads its whole halo from the host instead of NVLink peer copies")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline canvas of the last timed step to DIR/canvas.npy (float32; a fixed, seeded "
+                         f"sample of rows where the canvas exceeds {DUMP_BYTES >> 20} MiB), to compare two builds; "
+                         "--impl ours only: the reference arm times CPU code (the upstream implementation, or the "
+                         "oracle restatement where that is absent), not the CUDA path two builds differ in")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the canvas of the CUDA path (--impl ours); the reference arm runs CPU code")
     cfg = CONFIGS[args.config]
     # stdout carries exactly ONE JSON line: libraries that write to file descriptor 1 (NCCL prints its version banner
     # there under torchrun) are sent to stderr; the JSON line is written to the saved descriptor.

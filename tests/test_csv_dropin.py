@@ -83,29 +83,41 @@ def test_csv_reader_tolerant_fields_and_rejected_inputs(tmp_path, built):
     assert r.returncode == 2 and "Failed to read csv file." in r.stdout
 
 
+def _read_output(path):
+    return np.array([[float(v) for v in ln.split(",")] for ln in path.read_text().strip().split("\n")])
+
+
 @pytest.mark.gpu
 def test_aai_main_driver_matches_the_reference_main(tmp_path, built):
-    from oracle import ref
+    """The driver against the reference's own outputs stored in tests/golden: the reference main's settings (150 ->
+    25.4 dpi, 1.5 deg) on a reduced image in fast mode and in area-average mode, and an isocentre outside the image;
+    and the shipped settings it runs without arguments against the oracle."""
+    from common import golden_source, load_golden
+    from oracle import port
 
-    if not ref.available:
-        pytest.skip("oracle/_ref/libaai_ref.so not present")
-    _write_input(tmp_path / "Test_film_dose.csv")
-    out = _run_reference_main(str(tmp_path))
-    assert out.returncode == 0
-    want_text = (tmp_path / "Test_film_dose_mod.csv").read_text()
-    os.rename(tmp_path / "Test_film_dose_mod.csv", tmp_path / "ref_mod.csv")
+    z, meta = load_golden()
     exe = _build(tmp_path, os.path.join(ROOT, "examples", "aai_main.cpp"), "aai_main", True)
-    mine = subprocess.run([exe], cwd=str(tmp_path), capture_output=True, text=True)  # no arguments: shipped settings
+    for name in ("fast_dpi_default", "dpi_default_15deg", "neg_angle_far_iso"):
+        case = next(c for c in meta["cases"] if c["name"] == name)
+        src = golden_source(case).astype(np.float64)
+        with open(tmp_path / f"{name}.csv", "w") as f:
+            for row in src:
+                f.write(",".join(repr(float(v)) for v in row) + "\n")
+        args = [case["src_res"], case["dst_res"], case["iso"][0], case["iso"][1], case["angle"], case["mode"]]
+        mine = subprocess.run([exe, f"{name}.csv"] + [str(a) for a in args], cwd=str(tmp_path), capture_output=True,
+                              text=True)
+        assert mine.returncode == 0 and "Run terminated correctly." in mine.stdout, mine.stdout[-500:]
+        got, want = _read_output(tmp_path / f"{name}_mod.csv"), z[name]
+        assert got.shape == want.shape, name
+        # fast mode sums the same values in a different order: identical up to the 6-digit text format
+        assert np.abs(got - want).max() <= 2e-5 * np.abs(want).max(), name
+        same = sum(np.array_equal(g, [float("%.6g" % v) for v in w]) for g, w in zip(got, want))
+        assert same >= 0.9 * len(want), name
+    # no arguments: Test_film_dose.csv with the shipped settings, fast mode
+    img = _write_input(tmp_path / "Test_film_dose.csv")
+    mine = subprocess.run([exe], cwd=str(tmp_path), capture_output=True, text=True)
     assert mine.returncode == 0 and "Run terminated correctly." in mine.stdout, mine.stdout[-500:]
-    got_text = (tmp_path / "Test_film_dose_mod.csv").read_text()
-    want = np.array([[float(v) for v in ln.split(",")] for ln in want_text.strip().split("\n")])
-    got = np.array([[float(v) for v in ln.split(",")] for ln in got_text.strip().split("\n")])
-    assert want.shape == got.shape
-    # fast mode sums the same values in a different order: identical up to the 6-digit text format
+    got = _read_output(tmp_path / "Test_film_dose_mod.csv")
+    st, want, _ = port.run(img, 150.0, 25.4, (455.0, 455.0), 1.5, mode=2)
+    assert st == 0 and got.shape == want.shape
     assert np.abs(got - want).max() <= 2e-5 * np.abs(want).max()
-    same = sum(a == b for a, b in zip(got_text.split("\n"), want_text.split("\n")))
-    assert same >= 0.9 * len(want_text.split("\n"))
-    # and the area-average mode through the same driver
-    mine = subprocess.run([exe, "Test_film_dose.csv", "150", "25.4", "455", "455", "1.5", "1"], cwd=str(tmp_path),
-                          capture_output=True, text=True)
-    assert mine.returncode == 0, mine.stdout[-300:]
