@@ -20,11 +20,11 @@ LIB_PATH = os.path.join(_HERE, "libaai_b200.so")  # (developer A/B tools assign 
 AAI_OK = 0
 ERR_RESOLUTION_XY, ERR_RESOLUTION_NONPOS, ERR_NO_ROWS, ERR_NO_COLUMNS = 1, 2, 3, 4
 ERR_ANGLE, ERR_ARGUMENT, ERR_CUDA, ERR_NO_DEVICE = 5, 6, 7, 8
-F64, F32, U8 = 0, 1, 2
+F64, F32, U8, U16 = 0, 1, 2, 3
 MODE_AREA_AVERAGE, MODE_FAST, MODE_AREA_AVERAGE_EXACT = 1, 2, 3
 ARITH_F64, ARITH_F32, ARITH_F32_STAGED, ARITH_F32_BINNED, ARITH_F32_RING = 0, 1, 2, 3, 4
 
-_NP_TO_AAI = {np.dtype(np.float64): F64, np.dtype(np.float32): F32, np.dtype(np.uint8): U8}
+_NP_TO_AAI = {np.dtype(np.float64): F64, np.dtype(np.float32): F32, np.dtype(np.uint8): U8, np.dtype(np.uint16): U16}
 _AAI_TO_NP = {v: k for k, v in _NP_TO_AAI.items()}
 
 
@@ -232,7 +232,7 @@ def last_host_timing() -> dict:
 
 def _host_image(arr: np.ndarray) -> Image:
     if arr.dtype not in _NP_TO_AAI:
-        raise TypeError(f"unsupported dtype {arr.dtype}; use float64, float32 or uint8")
+        raise TypeError(f"unsupported dtype {arr.dtype}; use float64, float32, uint8 or uint16")
     if arr.ndim == 2:
         h, w = arr.shape
         ch = 1
@@ -249,7 +249,7 @@ def tensor_image(t, y0: int = 0, height: Optional[int] = None) -> Image:
     """``aai_image`` view of a CUDA (or pinned host) torch tensor [rows, w] / [rows, w, c] holding rows y0.. of an image."""
     import torch
 
-    dt = {torch.float64: F64, torch.float32: F32, torch.uint8: U8}[t.dtype]
+    dt = {torch.float64: F64, torch.float32: F32, torch.uint8: U8, torch.uint16: U16}[t.dtype]
     if t.dim() == 2:
         rows, w = t.shape
         ch = 1
@@ -436,9 +436,14 @@ class AreaAverageInterpolation:
     """Operator with the reference's method names and argument meaning (Source.cpp:52-57, 584-586).
 
     ``src`` is ``[h, w]`` (the reference's ``IMG``; float64 reproduces it exactly) or, as an extension,
-    ``[h, w, c]`` interleaved channels / float32 / uint8.  Returns ``Result``: ``ok``/``message`` are the
+    ``[h, w, c]`` interleaved channels / float32 / uint8 / uint16.  Returns ``Result``: ``ok``/``message`` are the
     reference's ``pair<bool,string>``, ``dst`` its resized output image, ``dst_isocenter`` its out parameter
     (left at ``dst_isocenter_in`` when validation fails, like the reference).
+
+    ``arith=ARITH_F32`` for float32 / uint8 / uint16 images.  The result is float64 for float64 and uint16 sources and
+    under ``ARITH_F64``, else float32; ``out_dtype`` overrides that (a uint8 canvas takes any source but uint16, a uint16
+    canvas a uint16 source only; integer canvases are rounded half up and saturated).  uint16 sources go to the library
+    as they are (2 bytes per value), so ``out_dtype=np.uint16`` or ``np.float32`` keeps every buffer small.
     """
 
     def __init__(self, arith: int = ARITH_F64, devices: Optional[Sequence[int]] = None, out_dtype=None):
@@ -461,8 +466,10 @@ class AreaAverageInterpolation:
         if src.dtype not in _NP_TO_AAI:
             src = src.astype(np.float64)
         src = np.ascontiguousarray(src)
+        # (uint16 sources keep the float64 result they had when they were widened to float64 before the call)
         out_dtype = np.dtype(self.out_dtype) if self.out_dtype is not None else (
-            np.dtype(np.float64) if src.dtype == np.float64 or self.arith == ARITH_F64 else np.dtype(np.float32))
+            np.dtype(np.float64) if src.dtype in (np.float64, np.uint16) or self.arith == ARITH_F64
+            else np.dtype(np.float32))
         shape = (plan.dst_h, plan.dst_w) + ((src.shape[2],) if src.ndim == 3 else ())
         dst = np.empty(shape, dtype=out_dtype)
         if dst.size:

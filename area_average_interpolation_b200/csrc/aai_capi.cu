@@ -22,15 +22,6 @@ thread_local char g_error[512] = "";
 std::atomic<int64_t> g_launches{0};
 thread_local float g_h2d_ms = -1.f, g_kernel_ms = -1.f, g_d2h_ms = -1.f;
 
-size_t elem_size(int dtype) {
-    switch (dtype) {
-        case AAI_F64: return 8;
-        case AAI_F32: return 4;
-        case AAI_U8: return 1;
-        default: return 0;
-    }
-}
-
 int cuda_fail(cudaError_t e, const char *what) {
     aai_set_error("%s: %s (%s)", what, cudaGetErrorString(e), cudaGetErrorName(e));
     return (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver) ? AAI_ERR_NO_DEVICE : AAI_ERR_CUDA;
@@ -42,9 +33,9 @@ int cuda_fail(cudaError_t e, const char *what) {
     } while (0)
 
 bool image_ok(const aai_image *im) {
-    return im && im->data && elem_size(im->dtype) && im->channels >= 1 && im->channels <= 4 && im->width > 0 &&
+    return im && im->data && aai_elem_size(im->dtype) && im->channels >= 1 && im->channels <= 4 && im->width > 0 &&
            im->height > 0 && im->rows >= 0 && im->y0 >= 0 && im->y0 + im->rows <= im->height &&
-           im->pitch_bytes >= (int64_t)(im->width * im->channels * (int64_t)elem_size(im->dtype));
+           im->pitch_bytes >= (int64_t)(im->width * im->channels * (int64_t)aai_elem_size(im->dtype));
 }
 
 // grow-only per-device scratch images used by aai_run_host (avoids cudaMalloc/cudaFree per call)
@@ -101,6 +92,14 @@ int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 }  // namespace
 
 void aai_count_extra_launches(int n) { g_launches.fetch_add(n); }
+
+int aai_check_dtype_pair(const char *who, int src_dtype, int dst_dtype) {
+    if (aai_dtype_pair_ok(src_dtype, dst_dtype)) return AAI_OK;
+    aai_set_error("%s: a %s source cannot write a %s canvas (a uint16 canvas takes a uint16 source; a uint16 source "
+                  "writes float64, float32 or uint16 canvases)",
+                  who, aai_dtype_name(src_dtype), aai_dtype_name(dst_dtype));
+    return AAI_ERR_ARGUMENT;
+}
 
 void aai_set_error(const char *fmt, ...) {
     va_list ap;
@@ -215,7 +214,7 @@ int aai_device_count(void) {
 
 int aai_image_alloc(aai_image *img, int device, int64_t width, int64_t height, int64_t y0, int64_t rows,
                     int32_t dtype, int32_t channels) {
-    if (!img || !elem_size(dtype) || channels < 1 || channels > 4 || width <= 0 || height <= 0 || rows < 0 ||
+    if (!img || !aai_elem_size(dtype) || channels < 1 || channels > 4 || width <= 0 || height <= 0 || rows < 0 ||
         y0 < 0 || y0 + rows > height) {
         aai_set_error("aai_image_alloc: bad argument");
         return AAI_ERR_ARGUMENT;
@@ -229,7 +228,7 @@ int aai_image_alloc(aai_image *img, int device, int64_t width, int64_t height, i
     img->dtype = dtype;
     img->channels = channels;
     // rows start on 512-byte boundaries: satisfies TMA's 16-byte global stride rule and 128-bit accesses
-    img->pitch_bytes = round_up(width * channels * (int64_t)elem_size(dtype), 512);
+    img->pitch_bytes = round_up(width * channels * (int64_t)aai_elem_size(dtype), 512);
     const size_t bytes = (size_t)img->pitch_bytes * (size_t)(rows > 0 ? rows : 1);
     AAI_CUDA(cudaMalloc(&img->data, bytes));
     return AAI_OK;
@@ -261,7 +260,7 @@ static int copy_rows(const aai_image *dst, const aai_image *src, cudaMemcpyKind 
     }
     if (band->rows == 0) return AAI_OK;
     AAI_CUDA(cudaSetDevice(device));
-    const size_t row_bytes = (size_t)(band->width * band->channels) * elem_size(band->dtype);
+    const size_t row_bytes = (size_t)(band->width * band->channels) * aai_elem_size(band->dtype);
     const char *s = (const char *)src->data + (kind == cudaMemcpyHostToDevice ? (band->y0 - src->y0) * src->pitch_bytes : 0);
     char *d = (char *)dst->data + (kind == cudaMemcpyDeviceToHost ? (band->y0 - dst->y0) * dst->pitch_bytes : 0);
     // Both images dense (no padding between rows): one linear copy (faster DMA than a strided 2-D copy).  With padded
@@ -291,7 +290,7 @@ int aai_image_copy_rows(const aai_image *dst, const aai_image *src, int64_t y0, 
     }
     if (y1 == y0) return AAI_OK;
     AAI_CUDA(cudaSetDevice(device));
-    const size_t row_bytes = (size_t)(src->width * src->channels) * elem_size(src->dtype);
+    const size_t row_bytes = (size_t)(src->width * src->channels) * aai_elem_size(src->dtype);
     char *d = (char *)dst->data + (y0 - dst->y0) * dst->pitch_bytes;
     const char *s = (const char *)src->data + (y0 - src->y0) * src->pitch_bytes;
     if ((size_t)dst->pitch_bytes == row_bytes && (size_t)src->pitch_bytes == row_bytes)  // dense: one linear copy
@@ -340,6 +339,7 @@ int aai_run_device(const aai_plan *plan, int mode, int arith, const aai_image *s
                       (long long)plan->src_w, (long long)plan->src_h, (long long)plan->dst_w, (long long)plan->dst_h);
         return AAI_ERR_ARGUMENT;
     }
+    if (const int r = aai_check_dtype_pair("aai_run_device", src->dtype, dst->dtype)) return r;
     if (mode != AAI_MODE_AREA_AVERAGE && mode != AAI_MODE_FAST && mode != AAI_MODE_AREA_AVERAGE_EXACT) {
         aai_set_error("aai_run_device: interpolation mode must be 1, 2 or 3");
         return AAI_ERR_ARGUMENT;
@@ -381,6 +381,7 @@ static int check_host_images(const char *who, const aai_plan *plan, const aai_im
         aai_set_error("%s: host images do not match the plan", who);
         return AAI_ERR_ARGUMENT;
     }
+    if (const int r = aai_check_dtype_pair(who, src->dtype, dst->dtype)) return r;
     if (whole && (src->y0 != 0 || src->rows != src->height || dst->y0 != 0 || dst->rows != dst->height)) {
         aai_set_error("%s: whole host images expected", who);
         return AAI_ERR_ARGUMENT;
@@ -410,7 +411,7 @@ int aai_expand_device(const aai_plan *plan, const aai_image *src, const aai_imag
     AaiKernelParams kp = aai_make_kernel_params(*plan, *src, canvas, 0, 0);
     kp.dst = dst_mod->data;
     kp.dst_pitch = dst_mod->pitch_bytes;
-    const int e = aai_launch_expand(kp, (int)elem_size(src->dtype), stream);
+    const int e = aai_launch_expand(kp, (int)aai_elem_size(src->dtype), stream);
     if (e != (int)cudaSuccess) return cuda_fail((cudaError_t)e, "expand kernel launch");
     g_launches.fetch_add(1);
     return AAI_OK;
@@ -458,6 +459,8 @@ int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_im
         return AAI_ERR_ARGUMENT;
     }
     if (plan->status != AAI_OK) return plan->status;
+    for (int k = 0; k < n_images; ++k)
+        if (const int r = aai_check_dtype_pair("aai_run_device_batch", srcs[k].dtype, dsts[k].dtype)) return r;
     // One launch for the whole batch when the images form an equally strided stack of whole images: the separable TMA
     // kernel takes the stack as a rank-3 tensor (grid.y = image), every other kernel as grid.z = image.
     const aai_image &s0 = srcs[0], &d0 = dsts[0];
@@ -526,10 +529,10 @@ int aai_run_host_band(const aai_plan *plan, int mode, int arith, const aai_image
     aai_image dsrc = *src, ddst = *dst;
     dsrc.y0 = sy0;
     dsrc.rows = sy1 - sy0;
-    dsrc.pitch_bytes = round_up(src->width * src->channels * (int64_t)elem_size(src->dtype), 512);
+    dsrc.pitch_bytes = round_up(src->width * src->channels * (int64_t)aai_elem_size(src->dtype), 512);
     ddst.y0 = row0;
     ddst.rows = row1 - row0;
-    ddst.pitch_bytes = round_up(dst->width * dst->channels * (int64_t)elem_size(dst->dtype), 512);
+    ddst.pitch_bytes = round_up(dst->width * dst->channels * (int64_t)aai_elem_size(dst->dtype), 512);
     std::lock_guard<std::mutex> busy(g_ws[device < kMaxDevices ? device : 0].busy);
     Workspace *w = nullptr;
     r = workspace_get(device, (size_t)dsrc.pitch_bytes * (size_t)(dsrc.rows > 0 ? dsrc.rows : 1),
@@ -676,8 +679,8 @@ int aai_run_host_batch(const aai_plan *plan, int mode, int arith, const aai_imag
     // once its kernel (source buffers) resp. its download (canvas buffers) has finished.
     constexpr int kRing = 3;
     aai_image ds = srcs[0], dd = dsts[0];
-    ds.pitch_bytes = round_up(ds.width * ds.channels * (int64_t)elem_size(ds.dtype), 512);
-    dd.pitch_bytes = round_up(dd.width * dd.channels * (int64_t)elem_size(dd.dtype), 512);
+    ds.pitch_bytes = round_up(ds.width * ds.channels * (int64_t)aai_elem_size(ds.dtype), 512);
+    dd.pitch_bytes = round_up(dd.width * dd.channels * (int64_t)aai_elem_size(dd.dtype), 512);
     const size_t s_bytes = (size_t)ds.pitch_bytes * (size_t)ds.height, d_bytes = (size_t)dd.pitch_bytes * (size_t)dd.height;
     int per = (int)(((size_t)192 << 20) / (s_bytes + d_bytes));
     per = per < 1 ? 1 : (per > 16 ? 16 : per);

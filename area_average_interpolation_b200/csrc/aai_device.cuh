@@ -1,7 +1,8 @@
-// Device helpers shared by the kernel translation units (aai_kernels.cu, aai_kernels_f32.cu).
+// Device helpers shared by the kernel translation units (aai_kernels.cu, aai_kernels_f32.cu, ...).
 #ifndef AAI_DEVICE_CUH_
 #define AAI_DEVICE_CUH_
 
+#include <cuda.h>
 #include <cuda_runtime.h>
 
 #include <cfloat>
@@ -17,6 +18,36 @@ namespace aai_dev {
 // re-measured on the final kernel: 1.478 / 1.463 ms against 1.466 ms (profiles/r1_v17_ab_occupancy_tiles.txt).
 constexpr int TILE_W = AAI_TILE_W;
 constexpr int TILE_H = AAI_TILE_H;
+
+// Element types: the AAI_* code of a C++ element type and the element type of its TMA tensor maps (the separable TMA
+// kernel, the STAGED / RING overlap and fast-mode kernels).
+template <typename T>
+struct Elem;
+template <>
+struct Elem<double> {
+    static constexpr int dtype = AAI_F64;
+    static constexpr CUtensorMapDataType tmap = CU_TENSOR_MAP_DATA_TYPE_FLOAT64;
+};
+template <>
+struct Elem<float> {
+    static constexpr int dtype = AAI_F32;
+    static constexpr CUtensorMapDataType tmap = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+};
+template <>
+struct Elem<uint16_t> {
+    static constexpr int dtype = AAI_U16;
+    static constexpr CUtensorMapDataType tmap = CU_TENSOR_MAP_DATA_TYPE_UINT16;
+};
+template <>
+struct Elem<uint8_t> {
+    static constexpr int dtype = AAI_U8;
+    static constexpr CUtensorMapDataType tmap = CU_TENSOR_MAP_DATA_TYPE_UINT8;
+};
+// (source, canvas) pairs that are instantiated: the dispatchers skip the others at compile time (the C ABI refuses them)
+template <typename TI, typename TO>
+constexpr bool pair_ok() {
+    return aai_dtype_pair_ok(Elem<TI>::dtype, Elem<TO>::dtype);
+}
 
 template <typename T>
 struct SrcLoad;
@@ -36,6 +67,53 @@ struct SrcLoad<uint8_t> {
         return (double)__ldg((const uint8_t *)row + idx);
     }
 };
+template <>
+struct SrcLoad<uint16_t> {
+    static __device__ __forceinline__ double get(const void *row, int idx) {
+        return (double)__ldg((const uint16_t *)row + idx);
+    }
+};
+
+// 16-bit value -> float without the conversion unit: the value placed in the mantissa of 2^23, minus 2^23 (exact below
+// 2^23; one LOP3 + one FADD instead of an I2F, which issues at a quarter of the FP32 rate)
+#ifndef AAI_U16_CVT_MAGIC
+#define AAI_U16_CVT_MAGIC 1  // 0: I2F (A/B in profiles/)
+#endif
+__device__ __forceinline__ float u16_to_float(uint32_t v) {
+#if AAI_U16_CVT_MAGIC
+    return __int_as_float(0x4B000000u | v) - 8388608.0f;
+#else
+    return (float)v;
+#endif
+}
+template <typename TA, typename T>
+__device__ __forceinline__ TA to_arith(T v) {
+    return (TA)v;
+}
+template <>
+__device__ __forceinline__ float to_arith<float, uint16_t>(uint16_t v) {
+    return u16_to_float(v);
+}
+
+// FP32 kernels: one source element at a byte address, as float (exact for 8- and 16-bit values)
+template <typename T>
+struct LoadF;
+template <>
+struct LoadF<double> {
+    static __device__ __forceinline__ float get(const char *p) { return (float)__ldg((const double *)p); }
+};
+template <>
+struct LoadF<float> {
+    static __device__ __forceinline__ float get(const char *p) { return __ldg((const float *)p); }
+};
+template <>
+struct LoadF<uint8_t> {
+    static __device__ __forceinline__ float get(const char *p) { return (float)__ldg((const uint8_t *)p); }
+};
+template <>
+struct LoadF<uint16_t> {
+    static __device__ __forceinline__ float get(const char *p) { return u16_to_float(__ldg((const uint16_t *)p)); }
+};
 
 template <typename T>
 __device__ __forceinline__ void store_dst(void *row, int idx, double v);
@@ -53,6 +131,34 @@ __device__ __forceinline__ void store_dst<uint8_t>(void *row, int idx, double v)
     double r = floor(v + 0.5);
     r = fmin(fmax(r, 0.0), 255.0);
     ((uint8_t *)row)[idx] = (uint8_t)(int)r;
+}
+template <>
+__device__ __forceinline__ void store_dst<uint16_t>(void *row, int idx, double v) {
+    // the 8-bit rule with the 16-bit bound: round half up, saturate to [0,65535]
+    double r = floor(v + 0.5);
+    r = fmin(fmax(r, 0.0), 65535.0);
+    ((uint16_t *)row)[idx] = (uint16_t)(int)r;
+}
+
+// The same stores from an FP32 result (FP32 kernels).  Integer canvases: v + 0.5f is exact below 2^23 and larger values
+// saturate, so the result is the one store_dst gives for (double)v.
+template <typename T>
+__device__ __forceinline__ void store_f(void *row, int idx, float v);
+template <>
+__device__ __forceinline__ void store_f<double>(void *row, int idx, float v) {
+    ((double *)row)[idx] = (double)v;
+}
+template <>
+__device__ __forceinline__ void store_f<float>(void *row, int idx, float v) {
+    ((float *)row)[idx] = v;
+}
+template <>
+__device__ __forceinline__ void store_f<uint8_t>(void *row, int idx, float v) {
+    ((uint8_t *)row)[idx] = (uint8_t)__float2int_rd(fminf(fmaxf(v + 0.5f, 0.0f), 255.0f));  // round half up, saturate
+}
+template <>
+__device__ __forceinline__ void store_f<uint16_t>(void *row, int idx, float v) {
+    ((uint16_t *)row)[idx] = (uint16_t)__float2int_rd(fminf(fmaxf(v + 0.5f, 0.0f), 65535.0f));  // round half up, saturate
 }
 
 // Batched launches: gridDim.z = the images of an equally strided stack that share one plan (aai_run_device_batch);

@@ -57,6 +57,35 @@ struct AaiKernelParams {
     int32_t src_batch_rows, dst_batch_rows;      // the same in rows of the pitch (grid.z kernels; strides are whole rows)
 };
 
+// Bytes per element of an AAI_* element type, 0 for an unknown type: the one table every buffer size is taken from.
+inline size_t aai_elem_size(int dtype) {
+    switch (dtype) {
+        case AAI_F64: return 8;
+        case AAI_F32: return 4;
+        case AAI_U16: return 2;
+        case AAI_U8: return 1;
+        default: return 0;
+    }
+}
+inline const char *aai_dtype_name(int dtype) {
+    switch (dtype) {
+        case AAI_F64: return "float64";
+        case AAI_F32: return "float32";
+        case AAI_U16: return "uint16";
+        case AAI_U8: return "uint8";
+        default: return "unknown";
+    }
+}
+// The (source, canvas) element-type pairs the kernels are compiled for (include/aai.h): a 16-bit canvas takes a 16-bit
+// source only, a 16-bit source writes float or 16-bit canvases.  Keeps the number of instantiations bounded.
+inline constexpr bool aai_dtype_pair_ok(int src_dtype, int dst_dtype) {
+    if (dst_dtype == AAI_U16) return src_dtype == AAI_U16;
+    if (src_dtype == AAI_U16) return dst_dtype != AAI_U8;
+    return true;
+}
+// AAI_OK, or AAI_ERR_ARGUMENT with a message naming the refused pair (aai_last_error); no CUDA call
+int aai_check_dtype_pair(const char *who, int src_dtype, int dst_dtype);
+
 AaiKernelParams aai_make_kernel_params(const aai_plan &plan, const aai_image &src, const aai_image &dst,
                                        int64_t row0, int64_t row1);
 

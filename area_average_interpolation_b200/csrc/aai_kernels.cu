@@ -105,7 +105,7 @@ __global__ void __launch_bounds__(TILE_W *TILE_H) fast_kernel(const __grid_const
     for (int ch = 0; ch < NC; ++ch) store_dst<TO>(drow, x * NC + ch, count > 0 ? acc[ch] / (double)count : 0.0);
 }
 
-// FP32 arithmetic for float / 8-bit images.  The inside test is a discontinuous decision, so -- as in the FP32 overlap
+// FP32 arithmetic for float / integer images.  The inside test is a discontinuous decision, so -- as in the FP32 overlap
 // kernel -- the footprint centre is split into a lattice point and an FP32 fraction, the smallest margin of the decisive
 // comparisons is tracked, and a pixel with a margin inside the guard band is redone in FP64 (pixel_fast_f64).
 template <typename TI, typename TO, int NC>
@@ -149,13 +149,7 @@ __global__ void __launch_bounds__(TILE_W *TILE_H) fast_kernel_f32(const __grid_c
                 }
                 count += 1.0f;
 #pragma unroll
-                for (int ch = 0; ch < NC; ++ch) {
-                    float v;
-                    if (sizeof(TI) == 8) v = (float)__ldg((const double *)p + ch);
-                    else if (sizeof(TI) == 4) v = __ldg((const float *)p + ch);
-                    else v = (float)__ldg((const uint8_t *)p + ch);
-                    acc[ch] += v;
-                }
+                for (int ch = 0; ch < NC; ++ch) acc[ch] += LoadF<TI>::get(p + ch * (int)sizeof(TI));
             }
         }
     }
@@ -239,9 +233,10 @@ cudaError_t launch_dst(KernelKind kind, const AaiKernelParams &kp, int dst_dtype
     switch (dst_dtype) {
         case AAI_F64: return launch_channels<TI, double>(kind, kp, stream);
         case AAI_F32: return launch_channels<TI, float>(kind, kp, stream);
-        case AAI_U8: return launch_channels<TI, uint8_t>(kind, kp, stream);
-        default: return cudaErrorInvalidValue;
+        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_channels<TI, uint8_t>(kind, kp, stream); break;
+        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_channels<TI, uint16_t>(kind, kp, stream); break;
     }
+    return cudaErrorInvalidValue;
 }
 
 cudaError_t launch_any(KernelKind kind, const AaiKernelParams &kp, int src_dtype, int dst_dtype, cudaStream_t stream) {
@@ -249,6 +244,7 @@ cudaError_t launch_any(KernelKind kind, const AaiKernelParams &kp, int src_dtype
         case AAI_F64: return launch_dst<double>(kind, kp, dst_dtype, stream);
         case AAI_F32: return launch_dst<float>(kind, kp, dst_dtype, stream);
         case AAI_U8: return launch_dst<uint8_t>(kind, kp, dst_dtype, stream);
+        case AAI_U16: return launch_dst<uint16_t>(kind, kp, dst_dtype, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -308,6 +304,7 @@ int aai_launch_expand(const AaiKernelParams &kp, int elem_bytes, void *stream) {
         k.row0 = r0;
         switch (elem_bytes) {
             case 1: expand_kernel<uint8_t><<<grid, 256, 0, st>>>(k); break;
+            case 2: expand_kernel<uint16_t><<<grid, 256, 0, st>>>(k); break;
             case 4: expand_kernel<float><<<grid, 256, 0, st>>>(k); break;
             case 8: expand_kernel<double><<<grid, 256, 0, st>>>(k); break;
             default: return (int)cudaErrorInvalidValue;
@@ -319,7 +316,7 @@ int aai_launch_expand(const AaiKernelParams &kp, int elem_bytes, void *stream) {
 }
 
 int aai_launch_fast(const AaiKernelParams &kp, int arith, int src_dtype, int dst_dtype, void *stream) {
-    // FP32 arithmetic on request for float / 8-bit sources (the mean of 8-byte doubles stays in FP64)
+    // FP32 arithmetic on request for float / integer sources (the mean of 8-byte doubles stays in FP64)
     const uint64_t max_e = (uint64_t)(kp.mod_w > kp.mod_h ? kp.mod_w : kp.mod_h);
     const bool f32 = arith == AAI_ARITH_F32 && src_dtype != AAI_F64 && dst_dtype != AAI_F64 && max_e < (1u << 30);
     // unrolled kernel: at most floor(2 hb + ~1e-5) + 1 lattice points per axis lie within hb of a footprint centre

@@ -199,9 +199,10 @@ cudaError_t launch1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t strea
     switch (dst_dtype) {
         case AAI_F64: return launch2<TI, double>(kp, stream);
         case AAI_F32: return launch2<TI, float>(kp, stream);
-        case AAI_U8: return launch2<TI, uint8_t>(kp, stream);
-        default: return cudaErrorInvalidValue;
+        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch2<TI, uint8_t>(kp, stream); break;
+        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch2<TI, uint16_t>(kp, stream); break;
     }
+    return cudaErrorInvalidValue;
 }
 
 }  // namespace
@@ -215,6 +216,7 @@ int AAI_CAT(aai_launch_overlap_f64_n, AAI_MAXN)(const AaiKernelParams &kp, int s
         case AAI_F64: return (int)launch1<double>(kp, dst_dtype, st);
         case AAI_F32: return (int)launch1<float>(kp, dst_dtype, st);
         case AAI_U8: return (int)launch1<uint8_t>(kp, dst_dtype, st);
+        case AAI_U16: return (int)launch1<uint16_t>(kp, dst_dtype, st);
         default: return (int)cudaErrorInvalidValue;
     }
 }

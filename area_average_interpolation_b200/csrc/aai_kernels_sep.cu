@@ -23,6 +23,7 @@
 #include <atomic>
 #include <cstdio>
 #include <cstdlib>
+#include <type_traits>
 
 #include "aai_device.cuh"
 
@@ -304,14 +305,17 @@ __global__ void __launch_bounds__(SEP_BLOCK)
 #pragma unroll
                         for (int q = 0; q < NV; ++q)
 #pragma unroll
-                            for (int e = 0; e < VEC; ++e) hs += wv[q * VEC + e] * (TA)v[u][q][e];
+                            for (int e = 0; e < VEC; ++e) hs += wv[q * VEC + e] * to_arith<TA>(v[u][q][e]);
                         acc[u] += w[u][k] * hs;
                     }
                 }
 #pragma unroll
                 for (int u = 0; u < U; ++u) {
                     const TA out = sep_normalise<TA>(acc[u], sumx * w[u][MAXT]);
-                    if (yb + u * RG < ylim) store_dst<TO>(out_row, x, (double)out);
+                    if (yb + u * RG < ylim) {
+                        if constexpr (std::is_same<TA, float>::value) store_f<TO>(out_row, x, out);
+                        else store_dst<TO>(out_row, x, out);
+                    }
                     out_row += (int64_t)RG * kp.dst_pitch;
                 }
             }
@@ -371,15 +375,6 @@ struct TmapCache {
     CUtensorMap map;
 };
 
-template <typename TI>
-CUtensorMapDataType tmap_dtype();
-template <>
-CUtensorMapDataType tmap_dtype<double>() { return CU_TENSOR_MAP_DATA_TYPE_FLOAT64; }
-template <>
-CUtensorMapDataType tmap_dtype<float>() { return CU_TENSOR_MAP_DATA_TYPE_FLOAT32; }
-template <>
-CUtensorMapDataType tmap_dtype<uint8_t>() { return CU_TENSOR_MAP_DATA_TYPE_UINT8; }
-
 // returns cudaErrorNotSupported when the fast path does not apply (the caller then uses the direct-tap kernel)
 template <typename TI, typename TO, typename TA, int TW, int MAXT>
 cudaError_t launch_sep(const AaiKernelParams &kp, cudaStream_t stream) {
@@ -438,13 +433,13 @@ cudaError_t launch_sep(const AaiKernelParams &kp, cudaStream_t stream) {
     const int64_t batch_stride = batch > 1 ? kp.src_batch_stride : kp.src_pitch * (int64_t)kp.src_rows;
     if (batch_stride % 16 != 0) return cudaErrorNotSupported;
     static thread_local TmapCache cache;  // per kernel instantiation and host thread
-    const TmapKey key = {kp.src, kp.src_pitch, batch_stride, kp.src_w, kp.src_rows, batch, sp.bw, sp.bh, (int32_t)tmap_dtype<TI>()};
+    const TmapKey key = {kp.src, kp.src_pitch, batch_stride, kp.src_w, kp.src_rows, batch, sp.bw, sp.bh, (int32_t)Elem<TI>::tmap};
     if (!cache.valid || !(cache.key == key)) {
         const cuuint64_t gdim[3] = {(cuuint64_t)kp.src_w, (cuuint64_t)kp.src_rows, (cuuint64_t)batch};
         const cuuint64_t gstride[2] = {(cuuint64_t)kp.src_pitch, (cuuint64_t)batch_stride};
         const cuuint32_t box[3] = {(cuuint32_t)sp.bw, (cuuint32_t)sp.bh, 1};
         const cuuint32_t estr[3] = {1, 1, 1};
-        const CUresult r = enc(&cache.map, tmap_dtype<TI>(), 3, const_cast<void *>(kp.src), gdim, gstride, box, estr,
+        const CUresult r = enc(&cache.map, Elem<TI>::tmap, 3, const_cast<void *>(kp.src), gdim, gstride, box, estr,
                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
                                CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) {
@@ -491,9 +486,10 @@ cudaError_t launch_sep_dst(const AaiKernelParams &kp, int dst_dtype, cudaStream_
     switch (dst_dtype) {
         case AAI_F64: return launch_sep_shape<TI, double, TA>(kp, stream);
         case AAI_F32: return launch_sep_shape<TI, float, TA>(kp, stream);
-        case AAI_U8: return launch_sep_shape<TI, uint8_t, TA>(kp, stream);
-        default: return cudaErrorInvalidValue;
+        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_sep_shape<TI, uint8_t, TA>(kp, stream); break;
+        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_sep_shape<TI, uint16_t, TA>(kp, stream); break;
     }
+    return cudaErrorInvalidValue;
 }
 
 template <typename TA>
@@ -502,6 +498,7 @@ cudaError_t launch_sep_src(const AaiKernelParams &kp, int src_dtype, int dst_dty
         case AAI_F64: return launch_sep_dst<double, TA>(kp, dst_dtype, stream);
         case AAI_F32: return launch_sep_dst<float, TA>(kp, dst_dtype, stream);
         case AAI_U8: return launch_sep_dst<uint8_t, TA>(kp, dst_dtype, stream);
+        case AAI_U16: return launch_sep_dst<uint16_t, TA>(kp, dst_dtype, stream);
         default: return cudaErrorInvalidValue;
     }
 }
@@ -557,14 +554,14 @@ __global__ void __launch_bounds__(TILE_W *TILE_H)
         for (int k = 0; k < MAXT; ++k)
 #pragma unroll
             for (int ch = 0; ch < NC; ++ch)
-                hs[ch] += wx[k] * (float)__ldg(reinterpret_cast<const TI *>(rowp + coff[k]) + ch);
+                hs[ch] += wx[k] * to_arith<float>(__ldg(reinterpret_cast<const TI *>(rowp + coff[k]) + ch));
 #pragma unroll
         for (int ch = 0; ch < NC; ++ch) acc[ch] += wy[r] * hs[ch];
     }
     char *drow = (char *)kp.dst + (int64_t)(y - dst_row0(kp)) * kp.dst_pitch;
     const float total = sumx * sumy;
 #pragma unroll
-    for (int ch = 0; ch < NC; ++ch) store_dst<TO>(drow, x * NC + ch, (double)sep_normalise<float>(acc[ch], total));
+    for (int ch = 0; ch < NC; ++ch) store_f<TO>(drow, x * NC + ch, sep_normalise<float>(acc[ch], total));
 }
 
 template <typename TI, typename TO, int NC>
@@ -601,9 +598,10 @@ template <typename TI>
 cudaError_t launch_direct_dst(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
     switch (dst_dtype) {
         case AAI_F32: return launch_direct_ch<TI, float>(kp, stream);
-        case AAI_U8: return launch_direct_ch<TI, uint8_t>(kp, stream);
-        default: return cudaErrorNotSupported;  // double destinations keep FP64 arithmetic
+        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_direct_ch<TI, uint8_t>(kp, stream); break;
+        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_direct_ch<TI, uint16_t>(kp, stream); break;
     }
+    return cudaErrorNotSupported;  // double destinations keep FP64 arithmetic
 }
 
 }  // namespace
@@ -628,6 +626,7 @@ int aai_launch_separable_direct_f32(const AaiKernelParams &kp, int src_dtype, in
     switch (src_dtype) {
         case AAI_F32: return (int)launch_direct_dst<float>(kp, dst_dtype, st);
         case AAI_U8: return (int)launch_direct_dst<uint8_t>(kp, dst_dtype, st);
+        case AAI_U16: return (int)launch_direct_dst<uint16_t>(kp, dst_dtype, st);
         default: return (int)cudaErrorNotSupported;
     }
 }

@@ -47,7 +47,6 @@ struct Blob {
 #pragma pack(pop)
 static_assert(sizeof(Blob) <= AAI_PEER_BLOB_BYTES, "blob size");
 
-size_t elem_size(int dtype) { return dtype == AAI_F64 ? 8 : dtype == AAI_F32 ? 4 : dtype == AAI_U8 ? 1 : 0; }
 int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
 
 struct Remote {  // what this rank knows about rank p
@@ -149,7 +148,7 @@ int aai_peer_upload_chunks(int n) {
 
 int aai_peer_create(const aai_plan *plan, int32_t dtype, int32_t channels, int rank, int world_size, int device,
                     aai_peer **out) {
-    if (!plan || !out || !elem_size(dtype) || channels < 1 || channels > 4 || world_size < 1 || rank < 0 ||
+    if (!plan || !out || !aai_elem_size(dtype) || channels < 1 || channels > 4 || world_size < 1 || rank < 0 ||
         rank >= world_size) {
         aai_set_error("aai_peer_create: bad argument");
         return AAI_ERR_ARGUMENT;
@@ -231,7 +230,7 @@ int aai_peer_export(aai_peer *g, unsigned char blob[AAI_PEER_BLOB_BYTES]) {
     b.world = g->world;
     int64_t y0, y1;
     owned_rows(g->plan.src_h, g->world, g->rank, y0, y1);
-    b.n_chunks = chunk_count(y1 - y0, g->plan.src_w * g->channels * (int64_t)elem_size(g->dtype));
+    b.n_chunks = chunk_count(y1 - y0, g->plan.src_w * g->channels * (int64_t)aai_elem_size(g->dtype));
     b.pitch = g->full.pitch_bytes;
     PEER_CUDA(cudaIpcGetMemHandle(&b.mem, g->full.data));
     std::memcpy(b.shm_name, g->shm_name, sizeof b.shm_name);
@@ -247,7 +246,7 @@ int aai_peer_connect(aai_peer *g, const unsigned char *blobs) {
     }
     PEER_CUDA(cudaSetDevice(g->device));
     g->remote.assign((size_t)g->world, Remote());
-    const int64_t row_bytes = g->plan.src_w * g->channels * (int64_t)elem_size(g->dtype);
+    const int64_t row_bytes = g->plan.src_w * g->channels * (int64_t)aai_elem_size(g->dtype);
     for (int p = 0; p < g->world; ++p) {
         Blob b;
         std::memcpy(&b, blobs + (size_t)p * AAI_PEER_BLOB_BYTES, sizeof b);
@@ -302,6 +301,9 @@ int aai_peer_device_source(const aai_peer *g, aai_image *out) {
 
 int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const aai_image *hdst, void *stream,
                  int synchronize) {
+    // (the element-type pair first: refused alike on every rank, whatever the state of its group)
+    if (hsrc && hdst)
+        if (const int r = aai_check_dtype_pair("aai_peer_run", hsrc->dtype, hdst->dtype)) return r;
     if (!g || !g->connected || !hsrc || !hdst || !hsrc->data || !hdst->data) {
         aai_set_error("aai_peer_run: group not connected or null image");
         return AAI_ERR_ARGUMENT;
@@ -309,12 +311,12 @@ int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const 
     const aai_plan &plan = g->plan;
     int64_t oy0, oy1;
     owned_rows(plan.src_h, g->world, g->rank, oy0, oy1);
-    const int64_t row_bytes = plan.src_w * g->channels * (int64_t)elem_size(g->dtype);
-    const int64_t dst_row_bytes = plan.dst_w * g->channels * (int64_t)elem_size(hdst->dtype);
+    const int64_t row_bytes = plan.src_w * g->channels * (int64_t)aai_elem_size(g->dtype);
+    const int64_t dst_row_bytes = plan.dst_w * g->channels * (int64_t)aai_elem_size(hdst->dtype);
     if (hsrc->width != plan.src_w || hsrc->height != plan.src_h || hsrc->dtype != g->dtype ||
         hsrc->channels != g->channels || hsrc->y0 > oy0 || hsrc->y0 + hsrc->rows < oy1 ||
         hsrc->pitch_bytes < row_bytes || hdst->width != plan.dst_w || hdst->height != plan.dst_h ||
-        !elem_size(hdst->dtype) || hdst->channels != g->channels || hdst->y0 > g->row0 ||
+        !aai_elem_size(hdst->dtype) || hdst->channels != g->channels || hdst->y0 > g->row0 ||
         hdst->y0 + hdst->rows < g->row1 || hdst->pitch_bytes < dst_row_bytes) {
         aai_set_error("aai_peer_run: host images must hold the owned source rows [%lld,%lld) and the canvas band [%lld,%lld)",
                       (long long)oy0, (long long)oy1, (long long)g->row0, (long long)g->row1);

@@ -47,8 +47,14 @@ enum {
     AAI_ERR_NO_DEVICE = 8       /* no usable CUDA device (there is no CPU fallback) */
 };
 
-/* Element types of pitched images. */
-enum { AAI_F64 = 0, AAI_F32 = 1, AAI_U8 = 2 };
+/* Element types of pitched images.  AAI_U16 is unsigned 16-bit (film scans, CT slices).
+ * Supported (source, canvas) pairs: F64 / F32 / U8 sources write F64, F32 or U8 canvases; a U16 source writes F64, F32
+ * or U16 canvases, and a U16 canvas takes a U16 source only.  The run functions refuse the other four pairs
+ * (F64 / F32 / U8 -> U16, U16 -> U8) with AAI_ERR_ARGUMENT before any CUDA call.
+ * Integer canvases (the reference only knows doubles): the real-valued result is rounded half up and saturated,
+ * to [0, 255] for U8 and to [0, 65535] for U16.  Integer sources take the same kernels as float sources, FP32 ones
+ * with AAI_ARITH_F32 (16-bit values are exact in FP32). */
+enum { AAI_F64 = 0, AAI_F32 = 1, AAI_U8 = 2, AAI_U16 = 3 };
 
 /* Interpolation mode = the reference's `interpolationMode` user setting (Source.cpp:1534). */
 enum {
@@ -112,7 +118,7 @@ typedef struct aai_image {
     int64_t pitch_bytes;
     int64_t width, height; /* of the FULL image */
     int64_t y0, rows;      /* rows present in `data` */
-    int32_t dtype;         /* AAI_F64 / AAI_F32 / AAI_U8 */
+    int32_t dtype;         /* AAI_F64 / AAI_F32 / AAI_U8 / AAI_U16 */
     int32_t channels;      /* 1..4 interleaved channels sharing one geometry */
 } aai_image;
 
