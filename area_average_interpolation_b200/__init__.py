@@ -118,6 +118,9 @@ def lib() -> C.CDLL:
         L.aai_run_device_batch.restype = C.c_int
         L.aai_run_device_batch.argtypes = [C.POINTER(Plan), C.c_int, C.c_int, C.POINTER(Image), C.POINTER(Image),
                                            C.c_int, C.c_int, C.c_void_p]
+        L.aai_run_device_adjoint.restype = C.c_int
+        L.aai_run_device_adjoint.argtypes = [C.POINTER(Plan), C.c_int, C.POINTER(Image), C.POINTER(Image), C.c_int,
+                                             C.c_int, C.c_void_p]
         L.aai_run_host.restype = C.c_int
         L.aai_run_host.argtypes = [C.POINTER(Plan), C.c_int, C.c_int, C.POINTER(Image), C.POINTER(Image),
                                    C.POINTER(C.c_int), C.c_int]
@@ -332,6 +335,18 @@ def run_device_batch(plan: Plan, src_imgs: Sequence[Image], dst_imgs: Sequence[I
     _check(lib().aai_run_device_batch(C.byref(plan), int(mode), int(arith), sa, da, n, int(device), C.c_void_p(stream)))
 
 
+def run_device_adjoint(plan: Plan, canvas_imgs: Sequence[Image], src_imgs: Sequence[Image],
+                       mode: int = MODE_AREA_AVERAGE, device: int = 0, stream: int = 0) -> None:
+    """``aai_run_device_adjoint``: ``src_imgs[k]`` receives the transpose of the resampling operator (FP64 weights)
+    applied to ``canvas_imgs[k]``.  Whole float32 / float64 device images, the same type and channel count on both
+    sides; one launch per kernel for an equally strided stack."""
+    n = len(canvas_imgs)
+    if len(src_imgs) != n:
+        raise ValueError("run_device_adjoint: as many source images as canvas images")
+    ca, sa = (Image * max(n, 1))(*canvas_imgs), (Image * max(n, 1))(*src_imgs)
+    _check(lib().aai_run_device_adjoint(C.byref(plan), int(mode), ca, sa, n, int(device), C.c_void_p(stream)))
+
+
 def run_host(plan: Plan, src: np.ndarray, dst: np.ndarray, mode: int = MODE_AREA_AVERAGE, arith: int = ARITH_F64,
              devices: Optional[Sequence[int]] = None) -> None:
     """``aai_run_host``: the reference call with host buffers (H2D, kernels on per-device streams, D2H)."""
@@ -492,9 +507,20 @@ class AreaAverageInterpolation:
                          dstIsocenter)
 
 
+def __getattr__(name):
+    # the torch entry points live in torch_ops, which imports torch: loaded on first use, not at package import (and
+    # left out of __all__, so that `from area_average_interpolation_b200 import *` does not import torch either)
+    if name in ("resample", "resample_adjoint"):
+        from . import torch_ops
+
+        return getattr(torch_ops, name)
+    raise AttributeError(f"module {__name__!r} has no attribute {name!r}")
+
+
 __all__ = [
     "AreaAverageInterpolation", "Result", "Plan", "Image", "AaiError", "make_plan", "partition_rows",
-    "band_source_window", "covered_pixels", "device_count", "launch_count", "last_host_timing", "run_device", "run_device_batch", "expand_device", "measure_fp32_tflops", "image_alloc", "image_free", "image_upload", "image_download", "image_copy_rows",
+    "band_source_window", "covered_pixels", "device_count", "launch_count", "last_host_timing", "run_device", "run_device_batch", "run_device_adjoint",
+    "expand_device", "measure_fp32_tflops", "image_alloc", "image_free", "image_upload", "image_download", "image_copy_rows",
     "ipc_export", "ipc_open", "ipc_close",
     "run_host", "run_host_band", "run_host_batch", "PeerGroup", "tensor_image", "status_string", "last_error", "lib", "LIB_PATH",
 ]

@@ -452,6 +452,31 @@ int aai_measure_fp32_tflops(int device, double *tflops) {
     return rc;
 }
 
+// Equally strided stack of whole images that match the plan: srcs[k].data = srcs[0].data + k * sstride, dsts likewise,
+// same pitch, dtype and channel count, strides positive whole rows (the grid.z kernels address the stack as one tall
+// image) below 2^30 rows.  Shared by aai_run_device_batch and aai_run_device_adjoint.
+static bool whole_image_stack(const aai_plan *plan, const aai_image *srcs, const aai_image *dsts, int n_images,
+                              int64_t *sstride_out, int64_t *dstride_out) {
+    const aai_image &s0 = srcs[0], &d0 = dsts[0];
+    bool stack = n_images > 1 && image_ok(&s0) && image_ok(&d0) && s0.y0 == 0 && s0.rows == s0.height && d0.y0 == 0 &&
+                 d0.rows == d0.height && s0.width == plan->src_w && s0.height == plan->src_h &&
+                 d0.width == plan->dst_w && d0.height == plan->dst_h && s0.channels == d0.channels;
+    const int64_t sstride = stack ? (const char *)srcs[1].data - (const char *)s0.data : 0;
+    const int64_t dstride = stack ? (const char *)dsts[1].data - (const char *)d0.data : 0;
+    for (int k = 1; stack && k < n_images; ++k) {
+        const aai_image &a = srcs[k], &b = dsts[k];
+        stack = a.data == (const char *)s0.data + k * sstride && b.data == (char *)d0.data + k * dstride &&
+                a.pitch_bytes == s0.pitch_bytes && b.pitch_bytes == d0.pitch_bytes && a.dtype == s0.dtype &&
+                b.dtype == d0.dtype && a.width == s0.width && a.height == s0.height && a.y0 == 0 &&
+                a.rows == a.height && b.width == d0.width && b.height == d0.height && b.y0 == 0 &&
+                b.rows == b.height && a.channels == s0.channels && b.channels == d0.channels;
+    }
+    *sstride_out = sstride;
+    *dstride_out = dstride;
+    return stack && sstride > 0 && dstride > 0 && sstride % s0.pitch_bytes == 0 && dstride % d0.pitch_bytes == 0 &&
+           sstride / s0.pitch_bytes < (1 << 30) && dstride / d0.pitch_bytes < (1 << 30);
+}
+
 int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_image *srcs, const aai_image *dsts,
                          int n_images, int device, void *stream) {
     if (!plan || !srcs || !dsts || n_images <= 0) {
@@ -464,25 +489,11 @@ int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_im
     // One launch for the whole batch when the images form an equally strided stack of whole images: the separable TMA
     // kernel takes the stack as a rank-3 tensor (grid.y = image), every other kernel as grid.z = image.
     const aai_image &s0 = srcs[0], &d0 = dsts[0];
-    bool stack = n_images > 1 && image_ok(&s0) && image_ok(&d0) && s0.y0 == 0 && s0.rows == s0.height && d0.y0 == 0 &&
-                 d0.rows == d0.height && s0.width == plan->src_w && s0.height == plan->src_h &&
-                 d0.width == plan->dst_w && d0.height == plan->dst_h && s0.channels == d0.channels &&
-                 (mode == AAI_MODE_AREA_AVERAGE || mode == AAI_MODE_FAST || mode == AAI_MODE_AREA_AVERAGE_EXACT) &&
-                 (arith == AAI_ARITH_F64 || arith == AAI_ARITH_F32 || arith == AAI_ARITH_F32_STAGED ||
-                  arith == AAI_ARITH_F32_BINNED || arith == AAI_ARITH_F32_RING);
-    const int64_t sstride = stack ? (const char *)srcs[1].data - (const char *)s0.data : 0;
-    const int64_t dstride = stack ? (const char *)dsts[1].data - (const char *)d0.data : 0;
-    for (int k = 1; stack && k < n_images; ++k) {
-        const aai_image &a = srcs[k], &b = dsts[k];
-        stack = a.data == (const char *)s0.data + k * sstride && b.data == (char *)d0.data + k * dstride &&
-                a.pitch_bytes == s0.pitch_bytes && b.pitch_bytes == d0.pitch_bytes && a.dtype == s0.dtype &&
-                b.dtype == d0.dtype && a.width == s0.width && a.height == s0.height && a.y0 == 0 &&
-                a.rows == a.height && b.width == d0.width && b.height == d0.height && b.y0 == 0 &&
-                b.rows == b.height && a.channels == s0.channels && b.channels == d0.channels;
-    }
-    // (the grid.z kernels address the stack as one tall image: strides must be whole rows)
-    if (stack && sstride > 0 && dstride > 0 && sstride % s0.pitch_bytes == 0 && dstride % d0.pitch_bytes == 0 &&
-        sstride / s0.pitch_bytes < (1 << 30) && dstride / d0.pitch_bytes < (1 << 30)) {
+    const bool known = (mode == AAI_MODE_AREA_AVERAGE || mode == AAI_MODE_FAST || mode == AAI_MODE_AREA_AVERAGE_EXACT) &&
+                       (arith == AAI_ARITH_F64 || arith == AAI_ARITH_F32 || arith == AAI_ARITH_F32_STAGED ||
+                        arith == AAI_ARITH_F32_BINNED || arith == AAI_ARITH_F32_RING);
+    int64_t sstride = 0, dstride = 0;
+    if (known && whole_image_stack(plan, srcs, dsts, n_images, &sstride, &dstride)) {
         AAI_CUDA(cudaSetDevice(device));
         const int64_t srows = sstride / s0.pitch_bytes, drows = dstride / d0.pitch_bytes;
         // images per launch: grid.y / grid.z limit, and row indices of the stack must stay below 2^31
@@ -508,6 +519,109 @@ int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_im
         const int r = aai_run_device(plan, mode, arith, &srcs[k], &dsts[k], 0, plan->dst_h, device, stream);
         if (r != AAI_OK) return r;
     }
+    return AAI_OK;
+}
+
+// Host-side argument checks of aai_run_device_adjoint, in the order the header lists them; no CUDA call
+static int check_adjoint_args(const aai_plan *plan, int mode, const aai_image *canvas_grads, const aai_image *src_grads,
+                              int n_images) {
+    const char *who = "aai_run_device_adjoint";
+    if (!plan || !canvas_grads || !src_grads || n_images <= 0) {
+        aai_set_error("%s: null pointer or no images", who);
+        return AAI_ERR_ARGUMENT;
+    }
+    if (plan->status != AAI_OK) return plan->status;
+    if (mode != AAI_MODE_AREA_AVERAGE && mode != AAI_MODE_FAST && mode != AAI_MODE_AREA_AVERAGE_EXACT) {
+        aai_set_error("%s: interpolation mode must be 1, 2 or 3", who);
+        return AAI_ERR_ARGUMENT;
+    }
+    for (int k = 0; k < n_images; ++k) {
+        const aai_image &g = canvas_grads[k], &s = src_grads[k];
+        if (!g.data || !s.data) {
+            aai_set_error("%s: image %d has no data", who, k);
+            return AAI_ERR_ARGUMENT;
+        }
+        if ((g.dtype != AAI_F32 && g.dtype != AAI_F64) || (s.dtype != AAI_F32 && s.dtype != AAI_F64) ||
+            g.dtype != s.dtype) {
+            aai_set_error("%s: gradients are float32 or float64, the same on both sides (image %d: canvas %s, source %s)",
+                          who, k, aai_dtype_name(g.dtype), aai_dtype_name(s.dtype));
+            return AAI_ERR_ARGUMENT;
+        }
+        if (g.channels != s.channels) {
+            aai_set_error("%s: image %d: the canvas has %d channels, the source %d", who, k, (int)g.channels,
+                          (int)s.channels);
+            return AAI_ERR_ARGUMENT;
+        }
+        if (g.y0 != 0 || g.rows != g.height || s.y0 != 0 || s.rows != s.height) {
+            aai_set_error("%s: image %d: whole images expected (y0 = 0, rows = height)", who, k);
+            return AAI_ERR_ARGUMENT;
+        }
+        if (g.width != plan->dst_w || g.height != plan->dst_h || s.width != plan->src_w || s.height != plan->src_h ||
+            !image_ok(&g) || !image_ok(&s)) {
+            aai_set_error("%s: image %d does not match the plan (source %lldx%lld, canvas %lldx%lld, 1-4 channels, "
+                          "pitch >= row bytes)",
+                          who, k, (long long)plan->src_w, (long long)plan->src_h, (long long)plan->dst_w,
+                          (long long)plan->dst_h);
+            return AAI_ERR_ARGUMENT;
+        }
+    }
+    return AAI_OK;
+}
+
+int aai_run_device_adjoint(const aai_plan *plan, int mode, const aai_image *canvas_grads, const aai_image *src_grads,
+                           int n_images, int device, void *stream) {
+    if (const int r = check_adjoint_args(plan, mode, canvas_grads, src_grads, n_images)) return r;
+    AAI_CUDA(cudaSetDevice(device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const aai_image &s0 = src_grads[0], &g0 = canvas_grads[0];
+    AaiAdjointParams ap;
+    std::memset(&ap, 0, sizeof ap);
+    ap.kp = aai_make_kernel_params(*plan, s0, g0, 0, plan->dst_h);
+    ap.kp.quirk = mode == AAI_MODE_AREA_AVERAGE_EXACT ? 0 : 1;
+    // 1/S_p in stream-ordered scratch: two calls in flight on different streams never share it
+    const size_t rcp_bytes = (size_t)plan->dst_w * (size_t)plan->dst_h * sizeof(double);
+    AAI_CUDA(cudaMallocAsync((void **)&ap.rcp, rcp_bytes, st));
+    int e = (int)cudaSuccess;
+    const char *what = "adjoint normaliser launch";
+    for (int64_t a = 0; a < plan->dst_h && e == (int)cudaSuccess; a += AAI_MAX_ROWS_PER_LAUNCH) {
+        ap.row0 = (int32_t)a;
+        ap.row1 = (int32_t)(a + AAI_MAX_ROWS_PER_LAUNCH < plan->dst_h ? a + AAI_MAX_ROWS_PER_LAUNCH : plan->dst_h);
+        e = aai_launch_adjoint_norm(ap, mode, plan->axis_aligned, st);
+        if (e == (int)cudaSuccess) g_launches.fetch_add(1);
+    }
+    ap.inv_side = 1.0 / plan->side;
+    // gather over source rows, slab by slab; an equally strided stack is one launch per slab (grid.z = image).  Element
+    // type and channel count are those of image `first`: a stack shares them (whole_image_stack), a list may mix them.
+    auto gather = [&](int first, int n, int64_t canvas_stride, int64_t out_stride) {
+        ap.kp.channels = src_grads[first].channels;
+        ap.canvas = canvas_grads[first].data;
+        ap.canvas_pitch = canvas_grads[first].pitch_bytes;
+        ap.canvas_stride = canvas_stride;
+        ap.out = src_grads[first].data;
+        ap.out_pitch = src_grads[first].pitch_bytes;
+        ap.out_stride = out_stride;
+        for (int64_t a = 0; a < plan->src_h; a += AAI_MAX_ROWS_PER_LAUNCH) {
+            ap.row0 = (int32_t)a;
+            ap.row1 = (int32_t)(a + AAI_MAX_ROWS_PER_LAUNCH < plan->src_h ? a + AAI_MAX_ROWS_PER_LAUNCH : plan->src_h);
+            const int r = aai_launch_adjoint_gather(ap, mode, plan->axis_aligned, src_grads[first].dtype, n, st);
+            if (r != (int)cudaSuccess) return r;
+            g_launches.fetch_add(1);
+        }
+        return (int)cudaSuccess;
+    };
+    if (e == (int)cudaSuccess) {
+        what = "adjoint gather launch";
+        int64_t sstride = 0, cstride = 0;
+        if (whole_image_stack(plan, src_grads, canvas_grads, n_images, &sstride, &cstride)) {
+            for (int first = 0; first < n_images && e == (int)cudaSuccess; first += 65535)  // grid.z limit
+                e = gather(first, n_images - first < 65535 ? n_images - first : 65535, cstride, sstride);
+        } else {
+            for (int k = 0; k < n_images && e == (int)cudaSuccess; ++k) e = gather(k, 1, 0, 0);
+        }
+    }
+    const cudaError_t ef = cudaFreeAsync(ap.rcp, st);
+    if (e != (int)cudaSuccess) return cuda_fail((cudaError_t)e, what);
+    AAI_CUDA(ef);
     return AAI_OK;
 }
 

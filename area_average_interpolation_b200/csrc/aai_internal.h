@@ -118,6 +118,24 @@ int aai_launch_overlap_f64_n5(const AaiKernelParams &kp, int src_dtype, int dst_
 int aai_launch_overlap_f64_n6(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream);
 int aai_launch_overlap_f64_n8(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream);
 
+// aai_kernels_adj.cu: adjoint of the resampling operator (aai_run_device_adjoint).  `kp` carries the plan's geometry
+// (built with the source gradients as `src` and the canvas gradients as `dst`); the pointers below are what the kernels
+// read and write.
+struct AaiAdjointParams {
+    AaiKernelParams kp;
+    double *rcp;                 // [dst_h][dst_w]: 1/S_p of the forward, 0 where it writes 0
+    double inv_side;             // 1/L (the gather's inverse centre map; no FP64 division in the kernel)
+    const void *canvas;          // canvas gradients of image 0; image k at canvas + k * canvas_stride bytes
+    int64_t canvas_pitch, canvas_stride;
+    void *out;                   // source gradients, likewise
+    int64_t out_pitch, out_stride;
+    int32_t row0, row1;          // rows of this launch: canvas rows (normaliser) or source rows (gather)
+};
+// one launch each over rows [ap.row0, ap.row1) (at most AAI_MAX_ROWS_PER_LAUNCH); return the cudaError_t as int
+int aai_launch_adjoint_norm(const AaiAdjointParams &ap, int mode, int axis_aligned, void *stream);
+int aai_launch_adjoint_gather(const AaiAdjointParams &ap, int mode, int axis_aligned, int dtype, int n_images,
+                              void *stream);
+
 void aai_set_error(const char *fmt, ...);
 // aai_launch_count() bookkeeping for launchers that start more than the one kernel the C ABI glue counts per call
 void aai_count_extra_launches(int n);

@@ -211,6 +211,19 @@ int aai_run_device(const aai_plan *plan, int mode, int arith, const aai_image *s
 int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_image *srcs, const aai_image *dsts,
                          int n_images, int device, void *stream);
 
+/* Adjoint (transpose) of what aai_run_device computes for `plan` and `mode`, FP64 weights: src_grads[k] receives
+ * G = F^T canvas_grads[k].  Whole device images; F32 or F64, the same type and channel count on both sides.  Equally
+ * strided stacks are one launch of each kernel (the rule of aai_run_device_batch), other lists run image by image.
+ * Deterministic: bitwise the same for a stack and for per-image calls.  Asynchronous on `stream`.
+ *
+ * The forward is out[p] = sum_q A_pq v[src(q)] / S_p (S_p = sum_q A_pq, out = 0 where S_p <= DBL_EPSILON; fast mode:
+ * A_pq = 1 for the cells whose centre lies in the closed footprint).  The adjoint is
+ * G[s] = sum over the expanded cells q of s of sum_p (A_pq / S_p) g[p], with the weights of the FP64 forward; the
+ * gradient of an AAI_ARITH_F32 forward is exact only to that arithmetic's tolerance.  F^T applied to a canvas of ones
+ * is the coverage of each source pixel.  Scratch (8 bytes per canvas pixel) is allocated and freed in stream order. */
+int aai_run_device_adjoint(const aai_plan *plan, int mode, const aai_image *canvas_grads, const aai_image *src_grads,
+                           int n_images, int device, void *stream);
+
 /* The reference call end to end with HOST buffers: upload (each device gets its band's halo), kernels on
  * per-device streams, download.  `devices` = NULL / n_devices = 0 means device 0.  No NCCL: bands are
  * independent.  Blocks until dst is complete. */
