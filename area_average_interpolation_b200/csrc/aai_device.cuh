@@ -7,6 +7,7 @@
 
 #include <cfloat>
 #include <cstdint>
+#include <type_traits>
 
 #include "aai_cell.cuh"
 #include "aai_internal.h"
@@ -47,6 +48,54 @@ struct Elem<uint8_t> {
 template <typename TI, typename TO>
 constexpr bool pair_ok() {
     return aai_dtype_pair_ok(Elem<TI>::dtype, Elem<TO>::dtype);
+}
+
+// Host-side dispatch from run-time AAI_* codes and channel counts to template arguments.  Each kernel family names the
+// element types and channel counts it is compiled for; nothing outside those lists is instantiated.
+template <typename T>
+struct Tag {
+    using type = T;
+};
+template <typename... Ts>
+struct Types {};
+using AnyElem = Types<double, float, uint8_t, uint16_t>;
+using NarrowElem = Types<float, uint8_t, uint16_t>;  // FP32-only kernels: no double side
+
+// f(Tag<T>{}) for the T among Ts whose Elem<T>::dtype is `dtype`; `otherwise` when there is none
+template <typename... Ts, typename F>
+cudaError_t with_elem(Types<Ts...>, int dtype, cudaError_t otherwise, F &&f) {
+    cudaError_t e = otherwise;
+    ((dtype == Elem<Ts>::dtype && (e = f(Tag<Ts>{}), true)) || ...);
+    return e;
+}
+// f(Tag<TI>{}, Tag<TO>{}) for an instantiated pair (pair_ok) of Srcs x Dsts; `otherwise` for any other pair
+// (nested generic lambdas: decltype of a captured parameter is a reference, so the type is taken in the outer one)
+template <typename Srcs, typename Dsts, typename F>
+cudaError_t with_pair(int src_dtype, int dst_dtype, cudaError_t otherwise, F &&f) {
+    return with_elem(Srcs{}, src_dtype, otherwise, [&](auto ti) {
+        using TI = typename decltype(ti)::type;
+        return with_elem(Dsts{}, dst_dtype, otherwise, [&](auto to) {
+            using TO = typename decltype(to)::type;
+            if constexpr (pair_ok<TI, TO>())
+                return f(Tag<TI>{}, Tag<TO>{});
+            else
+                return otherwise;
+        });
+    });
+}
+// f(std::integral_constant<int, NC>{}) for nc among NCs; `otherwise` when it is not listed
+template <int... NCs, typename F>
+cudaError_t with_channels(int nc, cudaError_t otherwise, F &&f) {
+    cudaError_t e = otherwise;
+    ((nc == NCs && (e = f(std::integral_constant<int, NCs>{}), true)) || ...);
+    return e;
+}
+
+// grid of the one-thread-per-canvas-pixel kernels over rows [row0, row1): TILE_W x TILE_H pixels per CTA, one z slice
+// per image of a batch
+inline dim3 canvas_grid(const AaiKernelParams &kp) {
+    const int rows = kp.row1 - kp.row0;
+    return dim3((kp.dst_w + TILE_W - 1) / TILE_W, (rows + TILE_H - 1) / TILE_H, kp.batch > 1 ? kp.batch : 1);
 }
 
 template <typename T>

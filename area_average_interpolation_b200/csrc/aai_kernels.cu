@@ -202,51 +202,27 @@ __global__ void __launch_bounds__(256) fp32_peak_kernel(float *out, int iters, f
 
 enum KernelKind { K_OVERLAP, K_SEPARABLE, K_FAST, K_FAST_F32 };
 
-template <typename TI, typename TO, int NC>
-cudaError_t launch_typed(KernelKind kind, const AaiKernelParams &kp, cudaStream_t stream) {
-    const int rows = kp.row1 - kp.row0;
-    if (rows <= 0 || kp.dst_w <= 0) return cudaSuccess;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid((kp.dst_w + TILE_W - 1) / TILE_W, (rows + TILE_H - 1) / TILE_H, kp.batch > 1 ? kp.batch : 1);
-    switch (kind) {
-        case K_OVERLAP: overlap_kernel_f64<TI, TO, NC><<<grid, block, 0, stream>>>(kp); break;
-        case K_SEPARABLE: separable_kernel_f64<TI, TO, NC><<<grid, block, 0, stream>>>(kp); break;
-        case K_FAST: fast_kernel<TI, TO, NC><<<grid, block, 0, stream>>>(kp); break;
-        case K_FAST_F32: fast_kernel_f32<TI, TO, NC><<<grid, block, 0, stream>>>(kp); break;
-    }
+template <KernelKind KIND, typename TI, typename TO, int NC>
+cudaError_t launch_typed(const AaiKernelParams &kp, cudaStream_t stream) {
+    if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return cudaSuccess;
+    const dim3 grid = canvas_grid(kp), block(TILE_W, TILE_H);
+    if constexpr (KIND == K_OVERLAP) overlap_kernel_f64<TI, TO, NC><<<grid, block, 0, stream>>>(kp);
+    if constexpr (KIND == K_SEPARABLE) separable_kernel_f64<TI, TO, NC><<<grid, block, 0, stream>>>(kp);
+    if constexpr (KIND == K_FAST) fast_kernel<TI, TO, NC><<<grid, block, 0, stream>>>(kp);
+    if constexpr (KIND == K_FAST_F32) fast_kernel_f32<TI, TO, NC><<<grid, block, 0, stream>>>(kp);
     return cudaGetLastError();
 }
 
-template <typename TI, typename TO>
-cudaError_t launch_channels(KernelKind kind, const AaiKernelParams &kp, cudaStream_t stream) {
-    switch (kp.channels) {
-        case 1: return launch_typed<TI, TO, 1>(kind, kp, stream);
-        case 2: return launch_typed<TI, TO, 2>(kind, kp, stream);
-        case 3: return launch_typed<TI, TO, 3>(kind, kp, stream);
-        case 4: return launch_typed<TI, TO, 4>(kind, kp, stream);
-        default: return cudaErrorInvalidValue;
-    }
-}
-
-template <typename TI>
-cudaError_t launch_dst(KernelKind kind, const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    switch (dst_dtype) {
-        case AAI_F64: return launch_channels<TI, double>(kind, kp, stream);
-        case AAI_F32: return launch_channels<TI, float>(kind, kp, stream);
-        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_channels<TI, uint8_t>(kind, kp, stream); break;
-        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_channels<TI, uint16_t>(kind, kp, stream); break;
-    }
-    return cudaErrorInvalidValue;
-}
-
-cudaError_t launch_any(KernelKind kind, const AaiKernelParams &kp, int src_dtype, int dst_dtype, cudaStream_t stream) {
-    switch (src_dtype) {
-        case AAI_F64: return launch_dst<double>(kind, kp, dst_dtype, stream);
-        case AAI_F32: return launch_dst<float>(kind, kp, dst_dtype, stream);
-        case AAI_U8: return launch_dst<uint8_t>(kind, kp, dst_dtype, stream);
-        case AAI_U16: return launch_dst<uint16_t>(kind, kp, dst_dtype, stream);
-        default: return cudaErrorInvalidValue;
-    }
+// the rolled kernels: every instantiated (source, canvas) pair of Srcs x Dsts, 1-4 channels
+template <KernelKind KIND, typename Srcs, typename Dsts>
+cudaError_t launch_any(const AaiKernelParams &kp, int src_dtype, int dst_dtype, cudaStream_t stream) {
+    return with_pair<Srcs, Dsts>(src_dtype, dst_dtype, cudaErrorInvalidValue, [&](auto ti, auto to) {
+        using TI = typename decltype(ti)::type;
+        using TO = typename decltype(to)::type;
+        return with_channels<1, 2, 3, 4>(kp.channels, cudaErrorInvalidValue, [&](auto nc) {
+            return launch_typed<KIND, TI, TO, decltype(nc)::value>(kp, stream);
+        });
+    });
 }
 
 }  // namespace
@@ -276,7 +252,7 @@ int aai_launch_overlap(const AaiKernelParams &kp, int arith, int src_dtype, int 
         else if (n <= 8) e = aai_launch_overlap_f64_n8(kp, src_dtype, dst_dtype, stream);
         if (e != (int)cudaErrorNotSupported) return e;
     }
-    return (int)launch_any(K_OVERLAP, kp, src_dtype, dst_dtype, (cudaStream_t)stream);
+    return (int)launch_any<K_OVERLAP, AnyElem, AnyElem>(kp, src_dtype, dst_dtype, (cudaStream_t)stream);
 }
 int aai_probe_fp32(int blocks, int iters, float *scratch, double *flop, void *stream) {
     fp32_peak_kernel<<<blocks, 256, 0, (cudaStream_t)stream>>>(scratch, iters, 0.999f, 0.001f);
@@ -291,7 +267,7 @@ int aai_launch_separable(const AaiKernelParams &kp, int arith, int src_dtype, in
         e = aai_launch_separable_direct_f32(kp, src_dtype, dst_dtype, stream);
         if (e != (int)cudaErrorNotSupported) return e;
     }
-    return (int)launch_any(K_SEPARABLE, kp, src_dtype, dst_dtype, (cudaStream_t)stream);
+    return (int)launch_any<K_SEPARABLE, AnyElem, AnyElem>(kp, src_dtype, dst_dtype, (cudaStream_t)stream);
 }
 int aai_launch_expand(const AaiKernelParams &kp, int elem_bytes, void *stream) {
     if (kp.mod_w <= 0 || kp.mod_h <= 0) return (int)cudaSuccess;
@@ -331,5 +307,6 @@ int aai_launch_fast(const AaiKernelParams &kp, int arith, int src_dtype, int dst
         if (nf <= 5) return aai_launch_fast_f32_n6(kp, src_dtype, dst_dtype, stream);
         if (nf <= 7) return aai_launch_fast_f32_n8(kp, src_dtype, dst_dtype, stream);
     }
-    return (int)launch_any(f32 ? K_FAST_F32 : K_FAST, kp, src_dtype, dst_dtype, (cudaStream_t)stream);
+    if (f32) return (int)launch_any<K_FAST_F32, NarrowElem, NarrowElem>(kp, src_dtype, dst_dtype, (cudaStream_t)stream);
+    return (int)launch_any<K_FAST, AnyElem, AnyElem>(kp, src_dtype, dst_dtype, (cudaStream_t)stream);
 }

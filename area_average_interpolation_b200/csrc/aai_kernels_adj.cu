@@ -186,26 +186,15 @@ __global__ void __launch_bounds__(TILE_W *TILE_H) adjoint_gather_kernel(const __
     for (int ch = 0; ch < NC; ++ch) store_dst<T>(orow, sx * NC + ch, acc[ch]);
 }
 
-template <int KIND, typename T>
-cudaError_t gather_channels(const AaiAdjointParams &ap, dim3 grid, cudaStream_t st) {
-    const dim3 block(TILE_W, TILE_H);
-    switch (ap.kp.channels) {
-        case 1: adjoint_gather_kernel<KIND, T, 1><<<grid, block, 0, st>>>(ap); break;
-        case 2: adjoint_gather_kernel<KIND, T, 2><<<grid, block, 0, st>>>(ap); break;
-        case 3: adjoint_gather_kernel<KIND, T, 3><<<grid, block, 0, st>>>(ap); break;
-        case 4: adjoint_gather_kernel<KIND, T, 4><<<grid, block, 0, st>>>(ap); break;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-}
-
 template <int KIND>
 cudaError_t gather_typed(const AaiAdjointParams &ap, int dtype, dim3 grid, cudaStream_t st) {
-    switch (dtype) {
-        case AAI_F64: return gather_channels<KIND, double>(ap, grid, st);
-        case AAI_F32: return gather_channels<KIND, float>(ap, grid, st);
-        default: return cudaErrorInvalidValue;
-    }
+    return with_elem(Types<double, float>{}, dtype, cudaErrorInvalidValue, [&](auto t) {
+        using T = typename decltype(t)::type;
+        return with_channels<1, 2, 3, 4>(ap.kp.channels, cudaErrorInvalidValue, [&](auto nc) {
+            adjoint_gather_kernel<KIND, T, decltype(nc)::value><<<grid, dim3(TILE_W, TILE_H), 0, st>>>(ap);
+            return cudaGetLastError();
+        });
+    });
 }
 
 int adj_kind(int mode, int axis_aligned) {

@@ -535,10 +535,8 @@ __global__ void __launch_bounds__(TILE_W *TILE_H, AAI_F32_MIN_BLOCKS)
 
 template <typename TI, typename TO, int NC>
 cudaError_t launch3(const AaiKernelParams &kp, cudaStream_t stream) {
-    const int rows = kp.row1 - kp.row0;
-    if (rows <= 0 || kp.dst_w <= 0) return cudaSuccess;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid((kp.dst_w + TILE_W - 1) / TILE_W, (rows + TILE_H - 1) / TILE_H, kp.batch > 1 ? kp.batch : 1);
+    if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return cudaSuccess;
+    const dim3 grid = canvas_grid(kp), block(TILE_W, TILE_H);
     if (kp.scale == 1 && kp.quadrant == 0) {
         StageHost h;
         if (kp.staged == 1 && stage_prepare<TI, NC>(kp, (double)kp.ext32, h)) {
@@ -552,20 +550,6 @@ cudaError_t launch3(const AaiKernelParams &kp, cudaStream_t stream) {
     else
         overlap_kernel_f32<TI, TO, NC, ADDR_GENERAL><<<grid, block, 0, stream>>>(kp);
     return cudaGetLastError();
-}
-template <typename TI, typename TO>
-cudaError_t launch2(const AaiKernelParams &kp, cudaStream_t stream) {
-    return kp.channels == 1 ? launch3<TI, TO, 1>(kp, stream) : launch3<TI, TO, 3>(kp, stream);
-}
-template <typename TI>
-cudaError_t launch1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    switch (dst_dtype) {
-        case AAI_F64: return launch2<TI, double>(kp, stream);
-        case AAI_F32: return launch2<TI, float>(kp, stream);
-        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch2<TI, uint8_t>(kp, stream); break;
-        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch2<TI, uint16_t>(kp, stream); break;
-    }
-    return cudaErrorInvalidValue;
 }
 
 
@@ -878,10 +862,8 @@ __global__ void __launch_bounds__(TILE_W *TILE_H, 1024 / (TILE_W * TILE_H))
 
 template <typename TI, typename TO, int NC>
 cudaError_t launch_fast3(const AaiKernelParams &kp, cudaStream_t stream) {
-    const int rows = kp.row1 - kp.row0;
-    if (rows <= 0 || kp.dst_w <= 0) return cudaSuccess;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid((kp.dst_w + TILE_W - 1) / TILE_W, (rows + TILE_H - 1) / TILE_H, kp.batch > 1 ? kp.batch : 1);
+    if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return cudaSuccess;
+    const dim3 grid = canvas_grid(kp), block(TILE_W, TILE_H);
     if (kp.scale == 1 && kp.quadrant == 0) {
         StageHost h;
         if ((kp.staged == 1 || kp.staged == 3) && stage_prepare<TI, NC>(kp, (double)kp.shapef.hb + 1e-5, h)) {
@@ -918,22 +900,6 @@ cudaError_t launch_fast3(const AaiKernelParams &kp, cudaStream_t stream) {
     }
     return cudaGetLastError();
 }
-template <typename TI>
-cudaError_t launch_fast1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    const bool one = kp.channels == 1;
-    switch (dst_dtype) {  // (double destinations take the FP64 fast kernel)
-        case AAI_F32: return one ? launch_fast3<TI, float, 1>(kp, stream) : launch_fast3<TI, float, 3>(kp, stream);
-        case AAI_U8:
-            if constexpr (pair_ok<TI, uint8_t>())
-                return one ? launch_fast3<TI, uint8_t, 1>(kp, stream) : launch_fast3<TI, uint8_t, 3>(kp, stream);
-            break;
-        case AAI_U16:
-            if constexpr (pair_ok<TI, uint16_t>())
-                return one ? launch_fast3<TI, uint16_t, 1>(kp, stream) : launch_fast3<TI, uint16_t, 3>(kp, stream);
-            break;
-    }
-    return cudaErrorInvalidValue;
-}
 
 }  // namespace
 
@@ -941,23 +907,23 @@ cudaError_t launch_fast1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t 
 #define AAI_CAT(a, b) AAI_CAT2(a, b)
 
 int AAI_CAT(aai_launch_overlap_f32_n, AAI_MAXN)(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (src_dtype) {
-        case AAI_F64: return (int)launch1<double>(kp, dst_dtype, st);
-        case AAI_F32: return (int)launch1<float>(kp, dst_dtype, st);
-        case AAI_U8: return (int)launch1<uint8_t>(kp, dst_dtype, st);
-        case AAI_U16: return (int)launch1<uint16_t>(kp, dst_dtype, st);
-        default: return (int)cudaErrorInvalidValue;
-    }
+    return (int)with_pair<AnyElem, AnyElem>(src_dtype, dst_dtype, cudaErrorInvalidValue, [&](auto ti, auto to) {
+        using TI = typename decltype(ti)::type;
+        using TO = typename decltype(to)::type;
+        return with_channels<1, 3>(kp.channels, cudaErrorInvalidValue, [&](auto nc) {
+            return launch3<TI, TO, decltype(nc)::value>(kp, (cudaStream_t)stream);
+        });
+    });
 }
 
-// fast mode, FP32 arithmetic: float / 8-bit / 16-bit sources, float or integer destinations, 1 or 3 channels
+// fast mode, FP32 arithmetic: float / 8-bit / 16-bit sources, float or integer destinations (double destinations take
+// the FP64 fast kernel), 1 or 3 channels
 int AAI_CAT(aai_launch_fast_f32_n, AAI_MAXN)(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (src_dtype) {
-        case AAI_F32: return (int)launch_fast1<float>(kp, dst_dtype, st);
-        case AAI_U8: return (int)launch_fast1<uint8_t>(kp, dst_dtype, st);
-        case AAI_U16: return (int)launch_fast1<uint16_t>(kp, dst_dtype, st);
-        default: return (int)cudaErrorInvalidValue;
-    }
+    return (int)with_pair<NarrowElem, NarrowElem>(src_dtype, dst_dtype, cudaErrorInvalidValue, [&](auto ti, auto to) {
+        using TI = typename decltype(ti)::type;
+        using TO = typename decltype(to)::type;
+        return with_channels<1, 3>(kp.channels, cudaErrorInvalidValue, [&](auto nc) {
+            return launch_fast3<TI, TO, decltype(nc)::value>(kp, (cudaStream_t)stream);
+        });
+    });
 }

@@ -176,33 +176,13 @@ __global__ void __launch_bounds__(TILE_W *TILE_H, AAI_F64_MIN_CTAS)
 
 template <typename TI, typename TO, int NC>
 cudaError_t launch3(const AaiKernelParams &kp, cudaStream_t stream) {
-    const int rows = kp.row1 - kp.row0;
-    if (rows <= 0 || kp.dst_w <= 0) return cudaSuccess;
-    dim3 block(TILE_W, TILE_H);
-    dim3 grid((kp.dst_w + TILE_W - 1) / TILE_W, (rows + TILE_H - 1) / TILE_H, kp.batch > 1 ? kp.batch : 1);
+    if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return cudaSuccess;
+    const dim3 grid = canvas_grid(kp), block(TILE_W, TILE_H);
     if (kp.scale == 1 && kp.quadrant == 0)
         overlap_kernel_f64u<TI, TO, NC, true><<<grid, block, 0, stream>>>(kp);
     else
         overlap_kernel_f64u<TI, TO, NC, false><<<grid, block, 0, stream>>>(kp);
     return cudaGetLastError();
-}
-template <typename TI, typename TO>
-cudaError_t launch2(const AaiKernelParams &kp, cudaStream_t stream) {
-    switch (kp.channels) {
-        case 1: return launch3<TI, TO, 1>(kp, stream);
-        case 3: return launch3<TI, TO, 3>(kp, stream);
-        default: return cudaErrorNotSupported;  // the caller falls back to the rolled kernel
-    }
-}
-template <typename TI>
-cudaError_t launch1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    switch (dst_dtype) {
-        case AAI_F64: return launch2<TI, double>(kp, stream);
-        case AAI_F32: return launch2<TI, float>(kp, stream);
-        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch2<TI, uint8_t>(kp, stream); break;
-        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch2<TI, uint16_t>(kp, stream); break;
-    }
-    return cudaErrorInvalidValue;
 }
 
 }  // namespace
@@ -210,13 +190,13 @@ cudaError_t launch1(const AaiKernelParams &kp, int dst_dtype, cudaStream_t strea
 #define AAI_CAT2(a, b) a##b
 #define AAI_CAT(a, b) AAI_CAT2(a, b)
 
+// 1 or 3 channels; cudaErrorNotSupported for other channel counts (the caller falls back to the rolled kernel)
 int AAI_CAT(aai_launch_overlap_f64_n, AAI_MAXN)(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream) {
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (src_dtype) {
-        case AAI_F64: return (int)launch1<double>(kp, dst_dtype, st);
-        case AAI_F32: return (int)launch1<float>(kp, dst_dtype, st);
-        case AAI_U8: return (int)launch1<uint8_t>(kp, dst_dtype, st);
-        case AAI_U16: return (int)launch1<uint16_t>(kp, dst_dtype, st);
-        default: return (int)cudaErrorInvalidValue;
-    }
+    return (int)with_pair<AnyElem, AnyElem>(src_dtype, dst_dtype, cudaErrorInvalidValue, [&](auto ti, auto to) {
+        using TI = typename decltype(ti)::type;
+        using TO = typename decltype(to)::type;
+        return with_channels<1, 3>(kp.channels, cudaErrorNotSupported, [&](auto nc) {
+            return launch3<TI, TO, decltype(nc)::value>(kp, (cudaStream_t)stream);
+        });
+    });
 }

@@ -481,26 +481,12 @@ cudaError_t launch_sep_shape(const AaiKernelParams &kp, cudaStream_t stream) {
     return e;
 }
 
-template <typename TI, typename TA>
-cudaError_t launch_sep_dst(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    switch (dst_dtype) {
-        case AAI_F64: return launch_sep_shape<TI, double, TA>(kp, stream);
-        case AAI_F32: return launch_sep_shape<TI, float, TA>(kp, stream);
-        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_sep_shape<TI, uint8_t, TA>(kp, stream); break;
-        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_sep_shape<TI, uint16_t, TA>(kp, stream); break;
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <typename TA>
-cudaError_t launch_sep_src(const AaiKernelParams &kp, int src_dtype, int dst_dtype, cudaStream_t stream) {
-    switch (src_dtype) {
-        case AAI_F64: return launch_sep_dst<double, TA>(kp, dst_dtype, stream);
-        case AAI_F32: return launch_sep_dst<float, TA>(kp, dst_dtype, stream);
-        case AAI_U8: return launch_sep_dst<uint8_t, TA>(kp, dst_dtype, stream);
-        case AAI_U16: return launch_sep_dst<uint16_t, TA>(kp, dst_dtype, stream);
-        default: return cudaErrorInvalidValue;
-    }
+// taps in TA arithmetic for the sources Srcs, every canvas type
+template <typename TA, typename Srcs>
+cudaError_t launch_sep_pair(const AaiKernelParams &kp, int src_dtype, int dst_dtype, cudaStream_t stream) {
+    return with_pair<Srcs, AnyElem>(src_dtype, dst_dtype, cudaErrorInvalidValue, [&](auto ti, auto to) {
+        return launch_sep_shape<typename decltype(ti)::type, typename decltype(to)::type, TA>(kp, stream);
+    });
 }
 
 
@@ -588,21 +574,6 @@ cudaError_t launch_direct_taps(const AaiKernelParams &kp, cudaStream_t stream) {
     }
     return cudaGetLastError();
 }
-template <typename TI, typename TO>
-cudaError_t launch_direct_ch(const AaiKernelParams &kp, cudaStream_t stream) {
-    if (kp.channels == 1) return launch_direct_taps<TI, TO, 1>(kp, stream);
-    if (kp.channels == 3) return launch_direct_taps<TI, TO, 3>(kp, stream);
-    return cudaErrorNotSupported;
-}
-template <typename TI>
-cudaError_t launch_direct_dst(const AaiKernelParams &kp, int dst_dtype, cudaStream_t stream) {
-    switch (dst_dtype) {
-        case AAI_F32: return launch_direct_ch<TI, float>(kp, stream);
-        case AAI_U8: if constexpr (pair_ok<TI, uint8_t>()) return launch_direct_ch<TI, uint8_t>(kp, stream); break;
-        case AAI_U16: if constexpr (pair_ok<TI, uint16_t>()) return launch_direct_ch<TI, uint16_t>(kp, stream); break;
-    }
-    return cudaErrorNotSupported;  // double destinations keep FP64 arithmetic
-}
 
 }  // namespace
 
@@ -612,21 +583,23 @@ int aai_launch_separable_tma(const AaiKernelParams &kp, int arith, int src_dtype
     if ((kp.src_pitch % 16) != 0 || (reinterpret_cast<uintptr_t>(kp.src) % 16) != 0) return (int)cudaErrorNotSupported;
     if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return (int)cudaSuccess;
     cudaStream_t st = (cudaStream_t)stream;
-    if (arith == AAI_ARITH_F32 && src_dtype != AAI_F64) return (int)launch_sep_src<float>(kp, src_dtype, dst_dtype, st);
-    return (int)launch_sep_src<double>(kp, src_dtype, dst_dtype, st);
+    if (arith == AAI_ARITH_F32 && src_dtype != AAI_F64)
+        return (int)launch_sep_pair<float, NarrowElem>(kp, src_dtype, dst_dtype, st);
+    return (int)launch_sep_pair<double, AnyElem>(kp, src_dtype, dst_dtype, st);
 }
 
 // FP32 direct-tap kernel for the axis-aligned cases the TMA kernel does not take (quadrants 1-3, scale > 1, RGB);
-// cudaErrorNotSupported -> the caller falls back to the FP64 direct-tap kernel.
+// cudaErrorNotSupported -> the caller falls back to the FP64 direct-tap kernel (also for double images, which keep FP64
+// arithmetic).
 int aai_launch_separable_direct_f32(const AaiKernelParams &kp, int src_dtype, int dst_dtype, void *stream) {
     const uint64_t max_e = (uint64_t)(kp.mod_w > kp.mod_h ? kp.mod_w : kp.mod_h);
     if (max_e * (uint64_t)kp.scale >= 0x100000000ULL) return (int)cudaErrorNotSupported;  // multiply-high division range
     if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return (int)cudaSuccess;
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (src_dtype) {
-        case AAI_F32: return (int)launch_direct_dst<float>(kp, dst_dtype, st);
-        case AAI_U8: return (int)launch_direct_dst<uint8_t>(kp, dst_dtype, st);
-        case AAI_U16: return (int)launch_direct_dst<uint16_t>(kp, dst_dtype, st);
-        default: return (int)cudaErrorNotSupported;
-    }
+    return (int)with_pair<NarrowElem, NarrowElem>(src_dtype, dst_dtype, cudaErrorNotSupported, [&](auto ti, auto to) {
+        using TI = typename decltype(ti)::type;
+        using TO = typename decltype(to)::type;
+        return with_channels<1, 3>(kp.channels, cudaErrorNotSupported, [&](auto nc) {
+            return launch_direct_taps<TI, TO, decltype(nc)::value>(kp, (cudaStream_t)stream);
+        });
+    });
 }

@@ -1,16 +1,13 @@
 #!/bin/bash
 # developer tool: build libaai_b200 variants with extra -D flags into csrc/gpurun_variants/<name>.so
 # usage: tools/build_variant.sh <name> [-DAAI_TILE_W=16 -DAAI_TILE_H=8 ...]
+# Sources and nvcc flags are the ones __graft_entry__.build() uses (build_library), plus the given flags.
 set -e
 name=$1; shift
 root=$(cd "$(dirname "$0")/.." && pwd)
 csrc=$root/area_average_interpolation_b200/csrc
 out=$csrc/gpurun_variants; tmp=$out/obj_$name; mkdir -p $tmp
-flags="-gencode arch=compute_100a,code=sm_100a -lineinfo -O3 -std=c++17 -Xcompiler -fPIC $*"
-pids=()
-for f in aai_plan.cpp aai_capi.cu aai_peer.cu aai_kernels.cu aai_kernels_sep.cu aai_kernels_bin.cu; do nvcc $flags -c $csrc/$f -o $tmp/${f%.*}.o & pids+=($!); done
-for n in 4 5 6 8; do nvcc $flags -DAAI_MAXN=$n -c $csrc/aai_kernels_f32.cu -o $tmp/f32_n$n.o & pids+=($!); nvcc $flags -DAAI_MAXN=$n -c $csrc/aai_kernels_f64.cu -o $tmp/f64_n$n.o & pids+=($!); done
-for p in "${pids[@]}"; do wait $p; done
-nvcc -shared -cudart static -o $out/$name.so $tmp/*.o
+python3 -c 'import sys; sys.path.insert(0, sys.argv[1]); import __graft_entry__ as g; g.build_library(sys.argv[2], sys.argv[3], sys.argv[4:])' \
+    "$root" "$out/$name.so" "$tmp" "$@"
 rm -rf $tmp
 echo built $out/$name.so
