@@ -38,6 +38,39 @@ bool image_ok(const aai_image *im) {
            im->pitch_bytes >= (int64_t)(im->width * im->channels * (int64_t)aai_elem_size(im->dtype));
 }
 
+// well-formed source and canvas images of the plan's sizes with one channel count (rows are the caller's business)
+bool images_match_plan(const aai_plan *plan, const aai_image *src, const aai_image *dst) {
+    return image_ok(src) && image_ok(dst) && src->width == plan->src_w && src->height == plan->src_h &&
+           dst->width == plan->dst_w && dst->height == plan->dst_h && src->channels == dst->channels;
+}
+bool mode_ok(int mode) { return mode >= AAI_MODE_AREA_AVERAGE && mode <= AAI_MODE_AREA_AVERAGE_EXACT; }
+bool arith_ok(int arith) { return arith >= AAI_ARITH_F64 && arith <= AAI_ARITH_F32_RING; }
+
+int check_plan(const char *who, const aai_plan *plan) {
+    if (plan) return plan->status;
+    aai_set_error("%s: null plan", who);
+    return AAI_ERR_ARGUMENT;
+}
+
+int check_device(const char *who, int device) {
+    if (aai_device_count() > device && device >= 0) return AAI_OK;
+    aai_set_error("%s: device %d not present; this library has no CPU fallback", who, device);
+    return aai_device_count() <= 0 ? AAI_ERR_NO_DEVICE : AAI_ERR_ARGUMENT;
+}
+
+// Launches fn(a, b) for each slab [a, b) of at most AAI_MAX_ROWS_PER_LAUNCH rows of [row0, row1), counting each
+// launch in aai_launch_count(): the kernels put rows on grid.y (<= 65535 CTAs), so taller row ranges (line scans, large
+// upscales) take several launches.  Returns the first launch error (cudaError_t as int).
+template <class Fn>
+int launch_slabs(int64_t row0, int64_t row1, Fn fn) {
+    for (int64_t a = row0; a < row1; a += AAI_MAX_ROWS_PER_LAUNCH) {
+        const int e = fn(a, a + AAI_MAX_ROWS_PER_LAUNCH < row1 ? a + AAI_MAX_ROWS_PER_LAUNCH : row1);
+        if (e != (int)cudaSuccess) return e;
+        g_launches.fetch_add(1);
+    }
+    return (int)cudaSuccess;
+}
+
 // grow-only per-device scratch images used by aai_run_host (avoids cudaMalloc/cudaFree per call)
 struct Workspace {
     void *ptr[2] = {nullptr, nullptr};
@@ -87,9 +120,76 @@ int workspace_get(int device, size_t bytes0, size_t bytes1, Workspace **out) {
     return AAI_OK;
 }
 
-int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
+// Head of a host-buffer run on `device`'s workspace: holds the workspace's busy lock in `busy` for the rest of the
+// run, sizes its buffers, picks the stream (the caller's, else the workspace's own) and records ev[0], the start of the
+// run.  A pipelined run asks for chunk_events > 0 chunk events and gets its copy streams forked off `st` at ev[0].
+int pipeline_head(std::unique_lock<std::mutex> &busy, int device, size_t bytes0, size_t bytes1, void *stream,
+                  int chunk_events, Workspace **out, cudaStream_t *st_out) {
+    busy = std::unique_lock<std::mutex>(g_ws[device < kMaxDevices ? device : 0].busy);
+    if (const int r = workspace_get(device, bytes0, bytes1, out)) return r;
+    Workspace *w = *out;
+    const cudaStream_t st = *st_out = stream ? (cudaStream_t)stream : w->stream;
+    // the workspace is shared by every run on this device: order this run after the previous one even when an
+    // asynchronous caller switched streams in between
+    if (w->done_valid) AAI_CUDA(cudaStreamWaitEvent(st, w->done, 0));
+    AAI_CUDA(aai_grow_events(w->chunk_ev, (size_t)chunk_events));
+    AAI_CUDA(cudaEventRecord(w->ev[0], st));
+    if (chunk_events > 0) {
+        AAI_CUDA(cudaStreamWaitEvent(w->up, w->ev[0], 0));
+        AAI_CUDA(cudaStreamWaitEvent(w->dn, w->ev[0], 0));
+    }
+    return AAI_OK;
+}
+
+// Tail of a host-buffer run: a pipelined run joins its copy streams back onto `st`; then ev[3] and `done` mark the end.
+// A synchronous call waits and stores aai_last_host_timing(): the three phases of an unpipelined run (ev[1] and ev[2]
+// between them), or the whole call of a pipelined one, whose overlapped phases cannot be separated.
+int pipeline_tail(Workspace *w, cudaStream_t st, bool pipelined, bool synchronize) {
+    if (pipelined) {
+        AAI_CUDA(cudaEventRecord(w->join_up, w->up));
+        AAI_CUDA(cudaEventRecord(w->join_dn, w->dn));
+        AAI_CUDA(cudaStreamWaitEvent(st, w->join_up, 0));
+        AAI_CUDA(cudaStreamWaitEvent(st, w->join_dn, 0));
+    }
+    AAI_CUDA(cudaEventRecord(w->ev[3], st));
+    AAI_CUDA(cudaEventRecord(w->done, st));
+    w->done_valid = true;
+    if (!synchronize) return AAI_OK;
+    AAI_CUDA(cudaStreamSynchronize(st));
+    if (!pipelined) {
+        AAI_CUDA(cudaEventElapsedTime(&g_h2d_ms, w->ev[0], w->ev[1]));
+        AAI_CUDA(cudaEventElapsedTime(&g_kernel_ms, w->ev[1], w->ev[2]));
+        AAI_CUDA(cudaEventElapsedTime(&g_d2h_ms, w->ev[2], w->ev[3]));
+        return AAI_OK;
+    }
+    float total = 0.f;
+    AAI_CUDA(cudaEventElapsedTime(&total, w->ev[0], w->ev[3]));
+    g_h2d_ms = total;
+    g_kernel_ms = 0.f;
+    g_d2h_ms = 0.f;
+    return AAI_OK;
+}
 
 }  // namespace
+
+cudaError_t aai_copy_pitched(void *dst, int64_t dst_pitch, const void *src, int64_t src_pitch, size_t row_bytes,
+                             int64_t rows, cudaMemcpyKind kind, cudaStream_t stream) {
+    if (rows <= 0) return cudaSuccess;
+    // Both sides dense (no padding between rows): one linear copy (faster DMA than a strided 2-D copy).  With padded
+    // rows the copy must not touch the bytes between rows -- a host image may be a column view of a wider array.
+    if ((size_t)dst_pitch == row_bytes && (size_t)src_pitch == row_bytes)
+        return cudaMemcpyAsync(dst, src, row_bytes * (size_t)rows, kind, stream);
+    return cudaMemcpy2DAsync(dst, (size_t)dst_pitch, src, (size_t)src_pitch, row_bytes, (size_t)rows, kind, stream);
+}
+
+cudaError_t aai_grow_events(std::vector<cudaEvent_t> &events, size_t n) {
+    while (events.size() < n) {
+        cudaEvent_t e;
+        if (const cudaError_t r = cudaEventCreateWithFlags(&e, cudaEventDisableTiming)) return r;
+        events.push_back(e);
+    }
+    return cudaSuccess;
+}
 
 void aai_count_extra_launches(int n) { g_launches.fetch_add(n); }
 
@@ -170,31 +270,22 @@ AaiKernelParams aai_make_kernel_params(const aai_plan &p, const aai_image &src, 
     return k;
 }
 
-// One kernel of the path over canvas rows [kp.row0, kp.row1): rows sit on grid.y (<= 65535 CTAs), so very tall row
-// ranges (line scans, large upscales) are cut into several launches; bands are independent, the result is the same.
+// One kernel of the path over canvas rows [kp.row0, kp.row1), slab by slab (bands are independent: the same result)
 static int launch_rows(const aai_plan &plan, int mode, int arith, AaiKernelParams kp, int src_dtype, int dst_dtype,
                        void *stream) {
-    const int32_t row0 = kp.row0, row1 = kp.row1;
     kp.staged = arith == AAI_ARITH_F32_STAGED ? 1 : arith == AAI_ARITH_F32_BINNED ? 2 : arith == AAI_ARITH_F32_RING ? 3 : 0;
     if (kp.staged) arith = AAI_ARITH_F32;
-    for (int64_t a = row0; a < row1; a += AAI_MAX_ROWS_PER_LAUNCH) {
+    return launch_slabs(kp.row0, kp.row1, [&](int64_t a, int64_t b) {
         kp.row0 = (int32_t)a;
-        kp.row1 = (int32_t)(a + AAI_MAX_ROWS_PER_LAUNCH < row1 ? a + AAI_MAX_ROWS_PER_LAUNCH : row1);
+        kp.row1 = (int32_t)b;
         {  // CTA row order: towards the end of the launch where the rotated image covers more of the canvas rows
             const int64_t n = kp.row1 - kp.row0, e = n / 8 > 64 ? 64 : (n / 8 > 0 ? n / 8 : 1);
             kp.reverse_rows = aai_covered_pixels(&plan, kp.row0, kp.row0 + e) > aai_covered_pixels(&plan, kp.row1 - e, kp.row1) ? 1 : 0;
         }
-        int e;
-        if (mode == AAI_MODE_FAST)
-            e = aai_launch_fast(kp, arith, src_dtype, dst_dtype, stream);
-        else if (plan.axis_aligned)
-            e = aai_launch_separable(kp, arith, src_dtype, dst_dtype, stream);
-        else
-            e = aai_launch_overlap(kp, arith, src_dtype, dst_dtype, stream);
-        if (e != (int)cudaSuccess) return e;
-        g_launches.fetch_add(1);
-    }
-    return (int)cudaSuccess;
+        if (mode == AAI_MODE_FAST) return aai_launch_fast(kp, arith, src_dtype, dst_dtype, stream);
+        if (plan.axis_aligned) return aai_launch_separable(kp, arith, src_dtype, dst_dtype, stream);
+        return aai_launch_overlap(kp, arith, src_dtype, dst_dtype, stream);
+    });
 }
 
 extern "C" {
@@ -227,8 +318,7 @@ int aai_image_alloc(aai_image *img, int device, int64_t width, int64_t height, i
     img->rows = rows;
     img->dtype = dtype;
     img->channels = channels;
-    // rows start on 512-byte boundaries: satisfies TMA's 16-byte global stride rule and 128-bit accesses
-    img->pitch_bytes = round_up(width * channels * (int64_t)aai_elem_size(dtype), 512);
+    img->pitch_bytes = aai_device_pitch(width, channels, dtype);
     const size_t bytes = (size_t)img->pitch_bytes * (size_t)(rows > 0 ? rows : 1);
     AAI_CUDA(cudaMalloc(&img->data, bytes));
     return AAI_OK;
@@ -263,13 +353,7 @@ static int copy_rows(const aai_image *dst, const aai_image *src, cudaMemcpyKind 
     const size_t row_bytes = (size_t)(band->width * band->channels) * aai_elem_size(band->dtype);
     const char *s = (const char *)src->data + (kind == cudaMemcpyHostToDevice ? (band->y0 - src->y0) * src->pitch_bytes : 0);
     char *d = (char *)dst->data + (kind == cudaMemcpyDeviceToHost ? (band->y0 - dst->y0) * dst->pitch_bytes : 0);
-    // Both images dense (no padding between rows): one linear copy (faster DMA than a strided 2-D copy).  With padded
-    // rows the copy must not touch the bytes between rows -- a host image may be a column view of a wider array.
-    if ((size_t)dst->pitch_bytes == row_bytes && (size_t)src->pitch_bytes == row_bytes)
-        AAI_CUDA(cudaMemcpyAsync(d, s, row_bytes * (size_t)band->rows, kind, (cudaStream_t)stream));
-    else
-        AAI_CUDA(cudaMemcpy2DAsync(d, (size_t)dst->pitch_bytes, s, (size_t)src->pitch_bytes, row_bytes,
-                                   (size_t)band->rows, kind, (cudaStream_t)stream));
+    AAI_CUDA(aai_copy_pitched(d, dst->pitch_bytes, s, src->pitch_bytes, row_bytes, band->rows, kind, (cudaStream_t)stream));
     return AAI_OK;
 }
 
@@ -293,11 +377,8 @@ int aai_image_copy_rows(const aai_image *dst, const aai_image *src, int64_t y0, 
     const size_t row_bytes = (size_t)(src->width * src->channels) * aai_elem_size(src->dtype);
     char *d = (char *)dst->data + (y0 - dst->y0) * dst->pitch_bytes;
     const char *s = (const char *)src->data + (y0 - src->y0) * src->pitch_bytes;
-    if ((size_t)dst->pitch_bytes == row_bytes && (size_t)src->pitch_bytes == row_bytes)  // dense: one linear copy
-        AAI_CUDA(cudaMemcpyAsync(d, s, row_bytes * (size_t)(y1 - y0), cudaMemcpyDefault, (cudaStream_t)stream));
-    else
-        AAI_CUDA(cudaMemcpy2DAsync(d, (size_t)dst->pitch_bytes, s, (size_t)src->pitch_bytes, row_bytes,
-                                   (size_t)(y1 - y0), cudaMemcpyDefault, (cudaStream_t)stream));
+    AAI_CUDA(aai_copy_pitched(d, dst->pitch_bytes, s, src->pitch_bytes, row_bytes, y1 - y0, cudaMemcpyDefault,
+                              (cudaStream_t)stream));
     return AAI_OK;
 }
 
@@ -328,24 +409,18 @@ int aai_ipc_close(void *device_ptr, int device) {
 
 int aai_run_device(const aai_plan *plan, int mode, int arith, const aai_image *src, const aai_image *dst,
                    int64_t row0, int64_t row1, int device, void *stream) {
-    if (!plan) {
-        aai_set_error("aai_run_device: null plan");
-        return AAI_ERR_ARGUMENT;
-    }
-    if (plan->status != AAI_OK) return plan->status;
-    if (!image_ok(src) || !image_ok(dst) || src->width != plan->src_w || src->height != plan->src_h ||
-        dst->width != plan->dst_w || dst->height != plan->dst_h || src->channels != dst->channels) {
+    if (const int r = check_plan("aai_run_device", plan)) return r;
+    if (!images_match_plan(plan, src, dst)) {
         aai_set_error("aai_run_device: images do not match the plan (src %lldx%lld, canvas %lldx%lld)",
                       (long long)plan->src_w, (long long)plan->src_h, (long long)plan->dst_w, (long long)plan->dst_h);
         return AAI_ERR_ARGUMENT;
     }
     if (const int r = aai_check_dtype_pair("aai_run_device", src->dtype, dst->dtype)) return r;
-    if (mode != AAI_MODE_AREA_AVERAGE && mode != AAI_MODE_FAST && mode != AAI_MODE_AREA_AVERAGE_EXACT) {
+    if (!mode_ok(mode)) {
         aai_set_error("aai_run_device: interpolation mode must be 1, 2 or 3");
         return AAI_ERR_ARGUMENT;
     }
-    if (arith != AAI_ARITH_F64 && arith != AAI_ARITH_F32 && arith != AAI_ARITH_F32_STAGED && arith != AAI_ARITH_F32_BINNED &&
-        arith != AAI_ARITH_F32_RING) {
+    if (!arith_ok(arith)) {
         aai_set_error("aai_run_device: unknown arithmetic %d", arith);
         return AAI_ERR_ARGUMENT;
     }
@@ -371,13 +446,8 @@ int aai_run_device(const aai_plan *plan, int mode, int arith, const aai_image *s
 
 static int check_host_images(const char *who, const aai_plan *plan, const aai_image *src, const aai_image *dst,
                              bool whole) {
-    if (!plan) {
-        aai_set_error("%s: null plan", who);
-        return AAI_ERR_ARGUMENT;
-    }
-    if (plan->status != AAI_OK) return plan->status;
-    if (!image_ok(src) || !image_ok(dst) || src->width != plan->src_w || src->height != plan->src_h ||
-        dst->width != plan->dst_w || dst->height != plan->dst_h || src->channels != dst->channels) {
+    if (const int r = check_plan(who, plan)) return r;
+    if (!images_match_plan(plan, src, dst)) {
         aai_set_error("%s: host images do not match the plan", who);
         return AAI_ERR_ARGUMENT;
     }
@@ -390,11 +460,7 @@ static int check_host_images(const char *who, const aai_plan *plan, const aai_im
 }
 
 int aai_expand_device(const aai_plan *plan, const aai_image *src, const aai_image *dst_mod, int device, void *stream) {
-    if (!plan) {
-        aai_set_error("aai_expand_device: null plan");
-        return AAI_ERR_ARGUMENT;
-    }
-    if (plan->status != AAI_OK) return plan->status;
+    if (const int r = check_plan("aai_expand_device", plan)) return r;
     if (!image_ok(src) || !image_ok(dst_mod) || src->width != plan->src_w || src->height != plan->src_h ||
         src->y0 != 0 || src->rows != src->height || dst_mod->width != plan->mod_w || dst_mod->height != plan->mod_h ||
         dst_mod->y0 != 0 || dst_mod->rows != dst_mod->height || src->dtype != dst_mod->dtype ||
@@ -458,9 +524,8 @@ int aai_measure_fp32_tflops(int device, double *tflops) {
 static bool whole_image_stack(const aai_plan *plan, const aai_image *srcs, const aai_image *dsts, int n_images,
                               int64_t *sstride_out, int64_t *dstride_out) {
     const aai_image &s0 = srcs[0], &d0 = dsts[0];
-    bool stack = n_images > 1 && image_ok(&s0) && image_ok(&d0) && s0.y0 == 0 && s0.rows == s0.height && d0.y0 == 0 &&
-                 d0.rows == d0.height && s0.width == plan->src_w && s0.height == plan->src_h &&
-                 d0.width == plan->dst_w && d0.height == plan->dst_h && s0.channels == d0.channels;
+    bool stack = n_images > 1 && images_match_plan(plan, &s0, &d0) && s0.y0 == 0 && s0.rows == s0.height &&
+                 d0.y0 == 0 && d0.rows == d0.height;
     const int64_t sstride = stack ? (const char *)srcs[1].data - (const char *)s0.data : 0;
     const int64_t dstride = stack ? (const char *)dsts[1].data - (const char *)d0.data : 0;
     for (int k = 1; stack && k < n_images; ++k) {
@@ -488,12 +553,10 @@ int aai_run_device_batch(const aai_plan *plan, int mode, int arith, const aai_im
         if (const int r = aai_check_dtype_pair("aai_run_device_batch", srcs[k].dtype, dsts[k].dtype)) return r;
     // One launch for the whole batch when the images form an equally strided stack of whole images: the separable TMA
     // kernel takes the stack as a rank-3 tensor (grid.y = image), every other kernel as grid.z = image.
+    // (An unknown mode or arithmetic takes the per-image path, where aai_run_device refuses it.)
     const aai_image &s0 = srcs[0], &d0 = dsts[0];
-    const bool known = (mode == AAI_MODE_AREA_AVERAGE || mode == AAI_MODE_FAST || mode == AAI_MODE_AREA_AVERAGE_EXACT) &&
-                       (arith == AAI_ARITH_F64 || arith == AAI_ARITH_F32 || arith == AAI_ARITH_F32_STAGED ||
-                        arith == AAI_ARITH_F32_BINNED || arith == AAI_ARITH_F32_RING);
     int64_t sstride = 0, dstride = 0;
-    if (known && whole_image_stack(plan, srcs, dsts, n_images, &sstride, &dstride)) {
+    if (mode_ok(mode) && arith_ok(arith) && whole_image_stack(plan, srcs, dsts, n_images, &sstride, &dstride)) {
         AAI_CUDA(cudaSetDevice(device));
         const int64_t srows = sstride / s0.pitch_bytes, drows = dstride / d0.pitch_bytes;
         // images per launch: grid.y / grid.z limit, and row indices of the stack must stay below 2^31
@@ -531,7 +594,7 @@ static int check_adjoint_args(const aai_plan *plan, int mode, const aai_image *c
         return AAI_ERR_ARGUMENT;
     }
     if (plan->status != AAI_OK) return plan->status;
-    if (mode != AAI_MODE_AREA_AVERAGE && mode != AAI_MODE_FAST && mode != AAI_MODE_AREA_AVERAGE_EXACT) {
+    if (!mode_ok(mode)) {
         aai_set_error("%s: interpolation mode must be 1, 2 or 3", who);
         return AAI_ERR_ARGUMENT;
     }
@@ -556,8 +619,7 @@ static int check_adjoint_args(const aai_plan *plan, int mode, const aai_image *c
             aai_set_error("%s: image %d: whole images expected (y0 = 0, rows = height)", who, k);
             return AAI_ERR_ARGUMENT;
         }
-        if (g.width != plan->dst_w || g.height != plan->dst_h || s.width != plan->src_w || s.height != plan->src_h ||
-            !image_ok(&g) || !image_ok(&s)) {
+        if (!images_match_plan(plan, &s, &g)) {
             aai_set_error("%s: image %d does not match the plan (source %lldx%lld, canvas %lldx%lld, 1-4 channels, "
                           "pitch >= row bytes)",
                           who, k, (long long)plan->src_w, (long long)plan->src_h, (long long)plan->dst_w,
@@ -581,14 +643,12 @@ int aai_run_device_adjoint(const aai_plan *plan, int mode, const aai_image *canv
     // 1/S_p in stream-ordered scratch: two calls in flight on different streams never share it
     const size_t rcp_bytes = (size_t)plan->dst_w * (size_t)plan->dst_h * sizeof(double);
     AAI_CUDA(cudaMallocAsync((void **)&ap.rcp, rcp_bytes, st));
-    int e = (int)cudaSuccess;
     const char *what = "adjoint normaliser launch";
-    for (int64_t a = 0; a < plan->dst_h && e == (int)cudaSuccess; a += AAI_MAX_ROWS_PER_LAUNCH) {
+    int e = launch_slabs(0, plan->dst_h, [&](int64_t a, int64_t b) {
         ap.row0 = (int32_t)a;
-        ap.row1 = (int32_t)(a + AAI_MAX_ROWS_PER_LAUNCH < plan->dst_h ? a + AAI_MAX_ROWS_PER_LAUNCH : plan->dst_h);
-        e = aai_launch_adjoint_norm(ap, mode, plan->axis_aligned, st);
-        if (e == (int)cudaSuccess) g_launches.fetch_add(1);
-    }
+        ap.row1 = (int32_t)b;
+        return aai_launch_adjoint_norm(ap, mode, plan->axis_aligned, st);
+    });
     ap.inv_side = 1.0 / plan->side;
     // gather over source rows, slab by slab; an equally strided stack is one launch per slab (grid.z = image).  Element
     // type and channel count are those of image `first`: a stack shares them (whole_image_stack), a list may mix them.
@@ -600,14 +660,11 @@ int aai_run_device_adjoint(const aai_plan *plan, int mode, const aai_image *canv
         ap.out = src_grads[first].data;
         ap.out_pitch = src_grads[first].pitch_bytes;
         ap.out_stride = out_stride;
-        for (int64_t a = 0; a < plan->src_h; a += AAI_MAX_ROWS_PER_LAUNCH) {
+        return launch_slabs(0, plan->src_h, [&](int64_t a, int64_t b) {
             ap.row0 = (int32_t)a;
-            ap.row1 = (int32_t)(a + AAI_MAX_ROWS_PER_LAUNCH < plan->src_h ? a + AAI_MAX_ROWS_PER_LAUNCH : plan->src_h);
-            const int r = aai_launch_adjoint_gather(ap, mode, plan->axis_aligned, src_grads[first].dtype, n, st);
-            if (r != (int)cudaSuccess) return r;
-            g_launches.fetch_add(1);
-        }
-        return (int)cudaSuccess;
+            ap.row1 = (int32_t)b;
+            return aai_launch_adjoint_gather(ap, mode, plan->axis_aligned, src_grads[first].dtype, n, st);
+        });
     };
     if (e == (int)cudaSuccess) {
         what = "adjoint gather launch";
@@ -634,30 +691,16 @@ int aai_run_host_band(const aai_plan *plan, int mode, int arith, const aai_image
         return AAI_ERR_ARGUMENT;
     }
     if (row1 == row0) return AAI_OK;
-    if (aai_device_count() <= device || device < 0) {
-        aai_set_error("aai_run_host_band: device %d not present; this library has no CPU fallback", device);
-        return aai_device_count() <= 0 ? AAI_ERR_NO_DEVICE : AAI_ERR_ARGUMENT;
-    }
+    if ((r = check_device("aai_run_host_band", device)) != AAI_OK) return r;
     int64_t sx0, sx1, sy0, sy1;
     aai_band_source_window(plan, row0, row1, &sx0, &sx1, &sy0, &sy1);
     aai_image dsrc = *src, ddst = *dst;
     dsrc.y0 = sy0;
     dsrc.rows = sy1 - sy0;
-    dsrc.pitch_bytes = round_up(src->width * src->channels * (int64_t)aai_elem_size(src->dtype), 512);
+    dsrc.pitch_bytes = aai_device_pitch(src->width, src->channels, src->dtype);
     ddst.y0 = row0;
     ddst.rows = row1 - row0;
-    ddst.pitch_bytes = round_up(dst->width * dst->channels * (int64_t)aai_elem_size(dst->dtype), 512);
-    std::lock_guard<std::mutex> busy(g_ws[device < kMaxDevices ? device : 0].busy);
-    Workspace *w = nullptr;
-    r = workspace_get(device, (size_t)dsrc.pitch_bytes * (size_t)(dsrc.rows > 0 ? dsrc.rows : 1),
-                      (size_t)ddst.pitch_bytes * (size_t)ddst.rows, &w);
-    if (r != AAI_OK) return r;
-    dsrc.data = w->ptr[0];
-    ddst.data = w->ptr[1];
-    cudaStream_t st = stream ? (cudaStream_t)stream : w->stream;
-    // the workspace is shared by every run on this device: order this run after the previous one even when an
-    // asynchronous caller switched streams in between
-    if (w->done_valid) AAI_CUDA(cudaStreamWaitEvent(st, w->done, 0));
+    ddst.pitch_bytes = aai_device_pitch(dst->width, dst->channels, dst->dtype);
     // Pipelined path for large bands: the canvas band is cut into chunks of rows; the source halo is uploaded
     // progressively (each source row once), chunk c's kernel starts as soon as its own halo has arrived and its rows
     // are downloaded while later chunks are still uploading / computing (PCIe is full duplex).  Three streams,
@@ -671,8 +714,15 @@ int aai_run_host_band(const aai_plan *plan, int mode, int arith, const aai_image
     if (const char *e = getenv("AAI_HOST_CHUNKS")) chunks = atoi(e) > 0 ? atoi(e) : chunks;
 #endif
     if (chunks > band_rows) chunks = (int)band_rows;
+    std::unique_lock<std::mutex> busy;
+    Workspace *w = nullptr;
+    cudaStream_t st = nullptr;
+    r = pipeline_head(busy, device, (size_t)dsrc.pitch_bytes * (size_t)(dsrc.rows > 0 ? dsrc.rows : 1),
+                      (size_t)ddst.pitch_bytes * (size_t)ddst.rows, stream, chunks > 1 ? 2 * chunks : 0, &w, &st);
+    if (r != AAI_OK) return r;
+    dsrc.data = w->ptr[0];
+    ddst.data = w->ptr[1];
     if (chunks <= 1) {
-        AAI_CUDA(cudaEventRecord(w->ev[0], st));
         if (dsrc.rows > 0) {
             r = aai_image_upload(&dsrc, src, device, st);
             if (r != AAI_OK) return r;
@@ -683,27 +733,9 @@ int aai_run_host_band(const aai_plan *plan, int mode, int arith, const aai_image
         AAI_CUDA(cudaEventRecord(w->ev[2], st));
         r = aai_image_download(dst, &ddst, device, st);
         if (r != AAI_OK) return r;
-        AAI_CUDA(cudaEventRecord(w->ev[3], st));
-        AAI_CUDA(cudaEventRecord(w->done, st));
-        w->done_valid = true;
-        if (synchronize || !stream) {
-            AAI_CUDA(cudaStreamSynchronize(st));
-            AAI_CUDA(cudaEventElapsedTime(&g_h2d_ms, w->ev[0], w->ev[1]));
-            AAI_CUDA(cudaEventElapsedTime(&g_kernel_ms, w->ev[1], w->ev[2]));
-            AAI_CUDA(cudaEventElapsedTime(&g_d2h_ms, w->ev[2], w->ev[3]));
-        }
-        return AAI_OK;
+        return pipeline_tail(w, st, false, synchronize || !stream);
     }
-    while ((int)w->chunk_ev.size() < 2 * chunks) {
-        cudaEvent_t e;
-        AAI_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        w->chunk_ev.push_back(e);
-    }
-    // fork: the three internal streams start after everything already queued on the caller's stream
-    AAI_CUDA(cudaEventRecord(w->ev[0], st));
     cudaStream_t s_k = st;  // kernels run on the caller's stream itself
-    AAI_CUDA(cudaStreamWaitEvent(w->up, w->ev[0], 0));
-    AAI_CUDA(cudaStreamWaitEvent(w->dn, w->ev[0], 0));
     int64_t have_lo = 0, have_hi = 0;  // source rows [have_lo, have_hi) already queued for upload
     bool have_any = false;
     auto upload_rows = [&](int64_t a, int64_t b) -> int {
@@ -750,24 +782,7 @@ int aai_run_host_band(const aai_plan *plan, int mode, int arith, const aai_image
         r = aai_image_download(dst, &part, device, w->dn);
         if (r != AAI_OK) return r;
     }
-    // join: the caller's stream continues after the last upload and the last download
-    AAI_CUDA(cudaEventRecord(w->join_up, w->up));
-    AAI_CUDA(cudaEventRecord(w->join_dn, w->dn));
-    AAI_CUDA(cudaStreamWaitEvent(st, w->join_up, 0));
-    AAI_CUDA(cudaStreamWaitEvent(st, w->join_dn, 0));
-    AAI_CUDA(cudaEventRecord(w->ev[3], st));
-    AAI_CUDA(cudaEventRecord(w->done, st));
-    w->done_valid = true;
-    if (synchronize || !stream) {
-        AAI_CUDA(cudaStreamSynchronize(st));
-        // overlapped phases cannot be separated: report the whole call as one figure
-        float total = 0.f;
-        AAI_CUDA(cudaEventElapsedTime(&total, w->ev[0], w->ev[3]));
-        g_h2d_ms = total;
-        g_kernel_ms = 0.f;
-        g_d2h_ms = 0.f;
-    }
-    return AAI_OK;
+    return pipeline_tail(w, st, true, synchronize || !stream);
 }
 
 int aai_run_host_batch(const aai_plan *plan, int mode, int arith, const aai_image *srcs, const aai_image *dsts,
@@ -784,36 +799,25 @@ int aai_run_host_batch(const aai_plan *plan, int mode, int arith, const aai_imag
             return AAI_ERR_ARGUMENT;
         }
     }
-    if (aai_device_count() <= device || device < 0) {
-        aai_set_error("aai_run_host_batch: device %d not present; this library has no CPU fallback", device);
-        return aai_device_count() <= 0 ? AAI_ERR_NO_DEVICE : AAI_ERR_ARGUMENT;
-    }
+    if (const int r = check_device("aai_run_host_batch", device)) return r;
     // Ring of kRing groups of `per` slices each in the device workspace: group i is uploaded (one copy per slice),
     // resampled with ONE batched launch and downloaded, on three streams; its buffers are reused by group i + kRing
     // once its kernel (source buffers) resp. its download (canvas buffers) has finished.
     constexpr int kRing = 3;
     aai_image ds = srcs[0], dd = dsts[0];
-    ds.pitch_bytes = round_up(ds.width * ds.channels * (int64_t)aai_elem_size(ds.dtype), 512);
-    dd.pitch_bytes = round_up(dd.width * dd.channels * (int64_t)aai_elem_size(dd.dtype), 512);
+    ds.pitch_bytes = aai_device_pitch(ds.width, ds.channels, ds.dtype);
+    dd.pitch_bytes = aai_device_pitch(dd.width, dd.channels, dd.dtype);
     const size_t s_bytes = (size_t)ds.pitch_bytes * (size_t)ds.height, d_bytes = (size_t)dd.pitch_bytes * (size_t)dd.height;
     int per = (int)(((size_t)192 << 20) / (s_bytes + d_bytes));
     per = per < 1 ? 1 : (per > 16 ? 16 : per);
     if (per > n_images) per = n_images;
     const int groups = (n_images + per - 1) / per;
-    std::lock_guard<std::mutex> busy(g_ws[device < kMaxDevices ? device : 0].busy);
+    std::unique_lock<std::mutex> busy;
     Workspace *w = nullptr;
-    int r = workspace_get(device, s_bytes * (size_t)per * kRing, d_bytes * (size_t)per * kRing, &w);
+    cudaStream_t st = nullptr;
+    int r = pipeline_head(busy, device, s_bytes * (size_t)per * kRing, d_bytes * (size_t)per * kRing, stream,
+                          3 * kRing, &w, &st);
     if (r != AAI_OK) return r;
-    cudaStream_t st = stream ? (cudaStream_t)stream : w->stream;
-    if (w->done_valid) AAI_CUDA(cudaStreamWaitEvent(st, w->done, 0));
-    while ((int)w->chunk_ev.size() < 3 * kRing) {
-        cudaEvent_t e;
-        AAI_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        w->chunk_ev.push_back(e);
-    }
-    AAI_CUDA(cudaEventRecord(w->ev[0], st));
-    AAI_CUDA(cudaStreamWaitEvent(w->up, w->ev[0], 0));
-    AAI_CUDA(cudaStreamWaitEvent(w->dn, w->ev[0], 0));
     std::vector<aai_image> gs((size_t)per), gd((size_t)per);
     for (int g = 0; g < groups; ++g) {
         const int slot = g % kRing, first = g * per, n = n_images - first < per ? n_images - first : per;
@@ -842,22 +846,7 @@ int aai_run_host_batch(const aai_plan *plan, int mode, int arith, const aai_imag
         }
         AAI_CUDA(cudaEventRecord(dn_done, w->dn));
     }
-    AAI_CUDA(cudaEventRecord(w->join_up, w->up));
-    AAI_CUDA(cudaEventRecord(w->join_dn, w->dn));
-    AAI_CUDA(cudaStreamWaitEvent(st, w->join_up, 0));
-    AAI_CUDA(cudaStreamWaitEvent(st, w->join_dn, 0));
-    AAI_CUDA(cudaEventRecord(w->ev[3], st));
-    AAI_CUDA(cudaEventRecord(w->done, st));
-    w->done_valid = true;
-    if (synchronize || !stream) {
-        AAI_CUDA(cudaStreamSynchronize(st));
-        float total = 0.f;
-        AAI_CUDA(cudaEventElapsedTime(&total, w->ev[0], w->ev[3]));
-        g_h2d_ms = total;
-        g_kernel_ms = 0.f;
-        g_d2h_ms = 0.f;
-    }
-    return AAI_OK;
+    return pipeline_tail(w, st, true, synchronize || !stream);
 }
 
 int aai_run_host(const aai_plan *plan, int mode, int arith, const aai_image *src, const aai_image *dst,

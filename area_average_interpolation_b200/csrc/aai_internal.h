@@ -2,6 +2,8 @@
 #ifndef AAI_INTERNAL_H_
 #define AAI_INTERNAL_H_
 
+#include <cuda_runtime.h>
+
 #include <cstdint>
 #include <vector>
 
@@ -66,6 +68,11 @@ inline size_t aai_elem_size(int dtype) {
         case AAI_U8: return 1;
         default: return 0;
     }
+}
+// Row pitch of the library's device images: rows start on 512-byte boundaries, which satisfies TMA's 16-byte global
+// stride rule and 128-bit accesses.
+inline int64_t aai_device_pitch(int64_t width, int32_t channels, int dtype) {
+    return (width * channels * (int64_t)aai_elem_size(dtype) + 511) / 512 * 512;
 }
 inline const char *aai_dtype_name(int dtype) {
     switch (dtype) {
@@ -139,5 +146,11 @@ int aai_launch_adjoint_gather(const AaiAdjointParams &ap, int mode, int axis_ali
 void aai_set_error(const char *fmt, ...);
 // aai_launch_count() bookkeeping for launchers that start more than the one kernel the C ABI glue counts per call
 void aai_count_extra_launches(int n);
+
+// Enqueues the copy of `rows` rows of `row_bytes` bytes between two pitched buffers; nothing for rows <= 0.
+cudaError_t aai_copy_pitched(void *dst, int64_t dst_pitch, const void *src, int64_t src_pitch, size_t row_bytes,
+                             int64_t rows, cudaMemcpyKind kind, cudaStream_t stream);
+// Creates timing-free events until `events` holds at least n (grow-only per-run event pools).
+cudaError_t aai_grow_events(std::vector<cudaEvent_t> &events, size_t n);
 
 #endif  // AAI_INTERNAL_H_

@@ -47,8 +47,6 @@ struct Blob {
 #pragma pack(pop)
 static_assert(sizeof(Blob) <= AAI_PEER_BLOB_BYTES, "blob size");
 
-int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
-
 struct Remote {  // what this rank knows about rank p
     void *full = nullptr;                 // p's device image, mapped here (nullptr for p == rank)
     PeerShm *shm = nullptr;
@@ -125,16 +123,6 @@ bool host_wait(const std::atomic<uint64_t> &v, uint64_t want) {
         }
     }
     return true;
-}
-
-int copy_rows_2d(void *dst, int64_t dst_pitch, const void *src, int64_t src_pitch, size_t row_bytes, int64_t rows,
-                 cudaMemcpyKind kind, cudaStream_t st) {
-    if (rows <= 0) return AAI_OK;
-    if ((size_t)dst_pitch == row_bytes && (size_t)src_pitch == row_bytes)
-        PEER_CUDA(cudaMemcpyAsync(dst, src, row_bytes * (size_t)rows, kind, st));
-    else
-        PEER_CUDA(cudaMemcpy2DAsync(dst, (size_t)dst_pitch, src, (size_t)src_pitch, row_bytes, (size_t)rows, kind, st));
-    return AAI_OK;
 }
 
 }  // namespace
@@ -361,10 +349,9 @@ int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const 
     for (int c = 0; c < me.n_chunks; ++c) {
         int64_t a, b;
         chunk_rows(oy0, oy1, me.n_chunks, c, a, b);
-        const int rc = copy_rows_2d((char *)g->full.data + a * g->full.pitch_bytes, g->full.pitch_bytes,
-                                    (const char *)hsrc->data + (a - hsrc->y0) * hsrc->pitch_bytes, hsrc->pitch_bytes,
-                                    (size_t)row_bytes, b - a, cudaMemcpyHostToDevice, g->up);
-        if (rc != AAI_OK) return rc;
+        PEER_CUDA(aai_copy_pitched((char *)g->full.data + a * g->full.pitch_bytes, g->full.pitch_bytes,
+                                   (const char *)hsrc->data + (a - hsrc->y0) * hsrc->pitch_bytes, hsrc->pitch_bytes,
+                                   (size_t)row_bytes, b - a, cudaMemcpyHostToDevice, g->up));
         PEER_CUDA(cudaEventRecord(g->landed[c], g->up));
     }
     PEER_CUDA(cudaEventRecord(g->t_up, g->up));
@@ -414,15 +401,10 @@ int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const 
                 a = std::max(a, g->halo_y0);
                 b = std::min(b, g->halo_y1);
                 if (b <= a) continue;
-                const int rc = copy_rows_2d((char *)g->full.data + a * g->full.pitch_bytes, g->full.pitch_bytes,
-                                            (const char *)r.full + a * g->full.pitch_bytes, g->full.pitch_bytes,
-                                            (size_t)row_bytes, b - a, cudaMemcpyDefault, g->pl);
-                if (rc != AAI_OK) return rc;
-                if (g->op_ev.size() <= n_pull) {
-                    cudaEvent_t e;
-                    PEER_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                    g->op_ev.push_back(e);
-                }
+                PEER_CUDA(aai_copy_pitched((char *)g->full.data + a * g->full.pitch_bytes, g->full.pitch_bytes,
+                                           (const char *)r.full + a * g->full.pitch_bytes, g->full.pitch_bytes,
+                                           (size_t)row_bytes, b - a, cudaMemcpyDefault, g->pl));
+                PEER_CUDA(aai_grow_events(g->op_ev, n_pull + 1));
                 PEER_CUDA(cudaEventRecord(g->op_ev[n_pull], g->pl));
                 ops.push_back({a, b, -1 - (int)n_pull});
                 ++n_pull;
@@ -444,11 +426,7 @@ int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const 
     const int64_t band_rows = g->row1 - g->row0;
     int chunks = band_rows >= 64 ? (int)std::min<int64_t>(8, band_rows / 16) : 1;
     if (band_rows <= 0) chunks = 0;
-    while ((int)g->k_ev.size() < chunks) {
-        cudaEvent_t e;
-        PEER_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        g->k_ev.push_back(e);
-    }
+    PEER_CUDA(aai_grow_events(g->k_ev, (size_t)chunks));
     std::vector<char> waited(ops.size(), 0);
     for (int j = 0; j < chunks; ++j) {
         const int64_t r0 = g->row0 + band_rows * j / chunks, r1 = g->row0 + band_rows * (j + 1) / chunks;
@@ -464,10 +442,9 @@ int aai_peer_run(aai_peer *g, int mode, int arith, const aai_image *hsrc, const 
         if (rc != AAI_OK) return rc;
         PEER_CUDA(cudaEventRecord(g->k_ev[(size_t)j], st));
         PEER_CUDA(cudaStreamWaitEvent(g->dn, g->k_ev[(size_t)j], 0));
-        const int rc2 = copy_rows_2d((char *)hdst->data + (r0 - hdst->y0) * hdst->pitch_bytes, hdst->pitch_bytes,
-                                     (const char *)g->band.data + (r0 - g->row0) * g->band.pitch_bytes,
-                                     g->band.pitch_bytes, (size_t)dst_row_bytes, r1 - r0, cudaMemcpyDeviceToHost, g->dn);
-        if (rc2 != AAI_OK) return rc2;
+        PEER_CUDA(aai_copy_pitched((char *)hdst->data + (r0 - hdst->y0) * hdst->pitch_bytes, hdst->pitch_bytes,
+                                   (const char *)g->band.data + (r0 - g->row0) * g->band.pitch_bytes,
+                                   g->band.pitch_bytes, (size_t)dst_row_bytes, r1 - r0, cudaMemcpyDeviceToHost, g->dn));
     }
     PEER_CUDA(cudaEventRecord(g->t_k, st));
     PEER_CUDA(cudaEventRecord(g->k_last, st));
