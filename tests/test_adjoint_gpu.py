@@ -67,6 +67,8 @@ GEOMS = (
     + [(21, 17, 1, r, a, (10.0, 8.0)) for r in (0.5, 1.7) for a in (0.0, 90.0, 180.0, 270.0)]
     + [(21, 17, 1, 0.37, 17.3, (-6.0, 25.0)), (21, 17, 1, 1.7, 197.3, (30.0, -4.0)), (21, 17, 1, 0.5, 270.0, (9.5, 7.5))]
     + [(16, 12, 3, 0.37, 30.0, (8.0, 6.0)), (16, 12, 3, 1.7, 45.0, (7.5, 5.5)), (16, 12, 3, 0.5, 0.0, (8.0, 6.0))]
+    + [(16, 12, 2, 0.37, 107.3, (8.0, 6.0)), (16, 12, 2, 1.7, 180.0, (7.5, 5.5))]
+    + [(16, 12, 4, 1.0, 61.0, (8.3, 5.8)), (16, 12, 4, 0.5, 270.0, (8.0, 6.0))]
 )
 _W = {}
 

@@ -824,18 +824,26 @@ def test_canvas_taller_than_the_grid_limit(aai, oracle):
     cut into several launches instead of failing."""
     import torch
 
-    w, h = 3, 530000
     rng = np.random.default_rng(6)
-    src = rng.uniform(0, 4096, size=(h, w)).astype(np.float32)
-    src_t = torch.from_numpy(src).cuda()
-    for angle, mode, arith in ((0.0, 1, aai.ARITH_F32), (0.0, 2, aai.ARITH_F32), (180.0, 1, aai.ARITH_F64)):
-        plan = aai.make_plan(w, h, 1.0, 1.0, (1.0, 265000.0), angle)
+    tall = rng.uniform(0, 4096, size=(530000, 3)).astype(np.float32)
+    wide = np.ascontiguousarray(tall.T)  # a quarter turn makes its canvas as tall
+    for angle, mode, arith in ((0.0, 1, aai.ARITH_F32), (0.0, 2, aai.ARITH_F32), (180.0, 1, aai.ARITH_F64),
+                               (90.0, 1, aai.ARITH_F32), (90.0, 2, aai.ARITH_F64), (270.0, 1, aai.ARITH_F64),
+                               (270.0, 2, aai.ARITH_F32)):
+        src = wide if angle in (90.0, 270.0) else tall
+        iso = (src.shape[1] / 2 - 0.5, src.shape[0] / 2)
+        plan = aai.make_plan(src.shape[1], src.shape[0], 1.0, 1.0, iso, angle)
         assert plan.status == 0 and plan.dst_h > 65535 * 8
+        # prefilled with NaN: a row that no slab writes fails below
+        out = torch.full((plan.dst_h, plan.dst_w), float("nan"), dtype=torch.float64, device="cuda")
         before = aai.launch_count()
-        out = _device_run(aai, plan, src_t, torch.float64, arith=arith, mode=mode)
+        aai.run_device(plan, aai.tensor_image(torch.from_numpy(src).cuda()), aai.tensor_image(out), mode=mode,
+                       arith=arith, stream=torch.cuda.current_stream().cuda_stream)
+        torch.cuda.synchronize()
         assert aai.launch_count() >= before + 2
+        assert not bool(out.isnan().any()), (angle, mode)
         for r0 in (0, 65535 * 8 - 2, plan.dst_h - 3):
-            st, want, _ = oracle.run(src, 1.0, 1.0, (1.0, 265000.0), angle, mode=mode, rows=(r0, r0 + 3))
+            st, want, _ = oracle.run(src, 1.0, 1.0, iso, angle, mode=mode, rows=(r0, r0 + 3))
             assert st == 0
             got = out[r0:r0 + 3].cpu().numpy()
             if mode == 2:  # centre-in ties at exactly symmetric geometry are decided by rounding noise (see fast-mode tests)
