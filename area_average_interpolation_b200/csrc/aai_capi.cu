@@ -238,6 +238,10 @@ AaiKernelParams aai_make_kernel_params(const aai_plan &p, const aai_image &src, 
     const double amp = std::fmax(1.0, std::fmax(g.inv_c, g.inv_s));
     const uint64_t max_e = (uint64_t)(p.mod_w > p.mod_h ? p.mod_w : p.mod_h);
     k.f32_ok = (s > 0.0 && c > 0.0 && amp <= 20.0 && max_e * p.scale < 0x100000000ULL) ? 1 : 0;
+    {
+        const int nmax = aai_f32_maxn(k.ext32);
+        k.tip_window = nmax > 0 && aai_tip_window_ok(c, s, p.side, nmax) ? 1 : 0;
+    }
     k.quirk = 1;
     k.reach = p.reach;
     k.hb = h * (c + s);

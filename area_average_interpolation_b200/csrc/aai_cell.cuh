@@ -182,6 +182,8 @@ struct AaiShapeF {
     float kq_s, kq_c;  // 1/(s L), 1/(c L)
     float qq_cs, qq_sc;  // c/(2 s), s/(2 c)
     float half_side;   // L/2
+    // tips of the footprint outside its cell window (aai_tip_strips_f32)
+    float tk_sc, tk_cs;  // s/(2c), c/(2s)
     int steep;   // 1: sin <= cos (major axis = y, the edges cross vertical grid lines rarely)
     int ncross;  // floor(L min(s,c)) + 1: most minor-axis grid lines one left/right edge can cross
 };
@@ -222,6 +224,8 @@ inline AaiShapeF aai_make_shape_f(double c, double s, double L) {
     g.qq_cs = (float)(c / (2.0 * s));
     g.qq_sc = (float)(s / (2.0 * c));
     g.half_side = (float)(L / 2);
+    g.tk_sc = (float)(s / (2.0 * c));
+    g.tk_cs = (float)(c / (2.0 * s));
     g.steep = s <= c ? 1 : 0;
     g.ncross = (int)floor(L * mn) + 1;
     return g;
@@ -311,6 +315,65 @@ AAI_HD AaiF2 aai_cell_exact_f32x2(const AaiShapeF &g, AaiF2 u0, AaiF2 v0, AaiF2 
     const AaiF2 aL = aai_fma2(ca, aai_f2(g.hc2), aai_fma2(cb, aai_f2(g.hs2), aai_f2(0.25f)));
     const AaiF2 half_br = aai_fma2(lenB, aai_f2(0.5f), aai_mul2(lenR, aai_f2(0.5f)));
     return aai_fma2(aT, aai_sub2(lenT, lenB), aai_fma2(aL, aai_sub2(lenL, lenR), half_br));
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// Cell window + tips.  Anchor a window of NW x NW cells at the first cell column and row a footprint box touches; what
+// of the footprint lies outside the window is its RIGHT tip F ∩ {x > window's right edge} and its BOTTOM tip
+// F ∩ {y > window's bottom edge}.  When aai_tip_window_ok holds for the shape and NW = nmax - 1, for every interior
+// footprint each tip is the triangle at the footprint's extreme vertex in x (resp. y), lies in the one cell column (row)
+// after the window, inside the window's rows (columns), and meets at most 3 of them; the two tips are disjoint.  So the
+// window's cells plus the strips of the two tips are the footprint's whole box, with the tip cells' exact areas.
+// ------------------------------------------------------------------------------------------------------------
+// Host, FP64, per plan: nmax = cells per axis the FP32 kernel is compiled for.  With D = L(c+s) the width of the footprint
+// box, the box starts up to one cell (+ the margin m for FP32 rounding of the cell range) before the footprint, so a tip
+// is at most w = D + 2 - nmax + m wide.  The right tip's lowest point, h(c-s) + w s/c, stays above the window's bottom
+// edge (nmax - 1 - hb - 1 - m from the centre at worst) iff w (c+s) <= L c s; the bottom tip's rightmost point gives the
+// same condition (this also keeps w below L min(c,s): the tip is bounded by the two edges at the vertex only).  Along the
+// strip axis a tip is w (c/s + s/c) long: at most 3 strips while that is below 2.
+inline bool aai_tip_window_ok(double c, double s, double L, int nmax) {
+    const double m = 1e-3;
+    const double D = L * (c + s);
+    const double w = D + 2.0 - nmax + m;
+    return c > 0.0 && s > 0.0 && D >= nmax - 2 + m && w < 1.0 - m && w * (c + s) <= L * c * s - m &&
+           w / (c * s) <= 2.0 - m;
+}
+
+// Device (and host tests): the tips of one footprint.  e0 / t0 = left / top boundary of the window, relative to the
+// centre.  Lane x: the right tip in window rows first[0] .. first[0] + 2, lane y: the bottom tip in window columns
+// first[1] .. first[1] + 2; area[j] = the tip's area in its strip first + j (indices clamped into 0 .. NW-1: strips
+// beyond the tip get 0).  Along the strip axis, at d from the vertex, a tip is w + k d wide on one side of the vertex and
+// w - d/k on the other (k = s/c for the right tip, c/s for the bottom one), so its area up to d is
+//     T(d) = a^2 / (2k) + (k/2) e (2w - e),   a = clamp(w + k d, 0, w),  e = clamp(d / k, 0, w),
+// and the strip [d_j, d_j+1] holds T(d_j+1) - T(d_j).  T is 0 at the strip boundary before the tip's near end (the first
+// strip is the one holding that end).  A footprint without a tip has w = 0, and every area is 0.  Branch-free; the two
+// tips share packed FP32 instructions.
+template <int NW>
+AAI_HD void aai_tip_strips_f32(const AaiShapeF &g, float e0, float t0, int (&first)[2], AaiF2 (&area)[3]) {
+    const AaiF2 o = aai_f2(t0, e0);           // strip boundary 0: top of window row 0, left of window column 0
+    const AaiF2 v = aai_f2(-g.y_lf, g.y_lf);  // the vertex along the strip axis: y = h(c-s) (right), x = h(s-c) (bottom)
+    const AaiF2 k = aai_f2(g.k_sc, g.k_cs), ki = aai_f2(g.k_cs, g.k_sc);
+    const AaiF2 hk = aai_f2(g.tk_sc, g.tk_cs), hki = aai_f2(g.tk_cs, g.tk_sc);
+    const AaiF2 wr = aai_sub2(aai_f2(g.hb - (float)NW), aai_f2(e0, t0));  // hb - the window's right / bottom edge
+    const AaiF2 w = aai_f2(fmaxf(wr.x, 0.0f), fmaxf(wr.y, 0.0f)), w2 = aai_add2(w, w);
+    const AaiF2 rel = aai_sub2(aai_fma2(w, aai_f2(-ki.x, -ki.y), v), o);  // the tip's near end, from boundary 0
+    int f0 = (int)floorf(rel.x), f1 = (int)floorf(rel.y);
+    f0 = f0 < 0 ? 0 : (f0 > NW - 1 ? NW - 1 : f0);
+    f1 = f1 < 0 ? 0 : (f1 > NW - 1 ? NW - 1 : f1);
+    first[0] = f0;
+    first[1] = f1;
+    const AaiF2 d0 = aai_add2(aai_sub2(o, v), aai_f2((float)f0, (float)f1));
+    AaiF2 prev = aai_f2(0.0f);
+#pragma unroll
+    for (int j = 0; j < 3; ++j) {
+        const AaiF2 d = aai_add2(d0, aai_f2((float)(j + 1)));
+        const AaiF2 a = aai_fma2(k, d, w), e = aai_mul2(d, ki);
+        const AaiF2 ac = aai_f2(fminf(fmaxf(a.x, 0.0f), w.x), fminf(fmaxf(a.y, 0.0f), w.y));
+        const AaiF2 ec = aai_f2(fminf(fmaxf(e.x, 0.0f), w.x), fminf(fmaxf(e.y, 0.0f), w.y));
+        const AaiF2 t = aai_fma2(aai_mul2(ac, ac), hki, aai_mul2(hk, aai_mul2(ec, aai_sub2(w2, ec))));
+        area[j] = aai_sub2(t, prev);
+        prev = t;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------------

@@ -35,6 +35,7 @@ struct AaiKernelParams {
                       // 2 = fast mode binned from the source side where aai_kernels_bin.cu applies (A/B variant),
                       // 3 = fast mode by the persistent, double-buffered staged kernel (A/B variant)
     int32_t reverse_rows;  // host side only: the launcher of short FP32 overlap launches picks the bottom-up instantiation
+    int32_t tip_window;    // host side only: aai_tip_window_ok for the plan's shape and aai_f32_maxn (FP32 overlap kernel)
     double reach;     // L*sqrt(2)/2 (search window, 426-429)
     double hb;        // h*(c+s): half extent of the footprint's axis-aligned bounding box
     int32_t mod_w, mod_h, dst_w, dst_h;
@@ -58,6 +59,13 @@ struct AaiKernelParams {
     int64_t src_batch_stride, dst_batch_stride;  // bytes between consecutive images
     int32_t src_batch_rows, dst_batch_rows;      // the same in rows of the pitch (grid.z kernels; strides are whole rows)
 };
+
+// Cells per axis of the FP32 overlap kernel's translation unit (4, 5, 6 or 8) for footprint boxes of half extent ext32:
+// at most floor(2 ext32) + 1 cells per axis have non-zero overlap; 0 when no unit holds them
+inline int aai_f32_maxn(float ext32) {
+    const int n = (int)floor(2.0 * (double)ext32 + 1e-6) + 1;  // = floor(2 hb + 1 + ~4e-6) + 1
+    return n <= 4 ? 4 : n <= 5 ? 5 : n <= 6 ? 6 : n <= 8 ? 8 : 0;
+}
 
 // Bytes per element of an AAI_* element type, 0 for an unknown type: the one table every buffer size is taken from.
 inline size_t aai_elem_size(int dtype) {

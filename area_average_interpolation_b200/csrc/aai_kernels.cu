@@ -229,12 +229,13 @@ cudaError_t launch_any(const AaiKernelParams &kp, int src_dtype, int dst_dtype, 
 
 int aai_launch_overlap(const AaiKernelParams &kp, int arith, int src_dtype, int dst_dtype, void *stream) {
     if (arith == AAI_ARITH_F32 && kp.f32_ok && (kp.channels == 1 || kp.channels == 3)) {
-        // at most floor(2*hb + 1) + 1 cells per axis have non-zero overlap
-        const int n = (int)floor(2.0 * (double)kp.ext32 + 1e-6) + 1;  // = floor(2 hb + 1 + ~4e-6) + 1
-        if (n <= 4) return aai_launch_overlap_f32_n4(kp, src_dtype, dst_dtype, stream);
-        if (n <= 5) return aai_launch_overlap_f32_n5(kp, src_dtype, dst_dtype, stream);
-        if (n <= 6) return aai_launch_overlap_f32_n6(kp, src_dtype, dst_dtype, stream);
-        if (n <= 8) return aai_launch_overlap_f32_n8(kp, src_dtype, dst_dtype, stream);
+        switch (aai_f32_maxn(kp.ext32)) {
+            case 4: return aai_launch_overlap_f32_n4(kp, src_dtype, dst_dtype, stream);
+            case 5: return aai_launch_overlap_f32_n5(kp, src_dtype, dst_dtype, stream);
+            case 6: return aai_launch_overlap_f32_n6(kp, src_dtype, dst_dtype, stream);
+            case 8: return aai_launch_overlap_f32_n8(kp, src_dtype, dst_dtype, stream);
+            default: break;
+        }
     }
     // FP64 arithmetic: the unrolled kernel when the footprint fits its register arrays, else the rolled one
     // (its general-frame addressing divides by the scale with a multiply-high, exact below 2^32 / scale)

@@ -38,6 +38,13 @@ constexpr int MAXN = AAI_MAXN;
 #define AAI_ROW_UNROLL 1
 #endif
 constexpr int kRowUnroll = AAI_ROW_UNROLL;
+#ifndef AAI_WIN_ROW_UNROLL
+// rows of the cell window (WIN below) per loop iteration: all of them.  Measured on config 4 (MAXN 5, B200 at 1000 W,
+// 1965 MHz): 1.314 ms with 1 row, 1.307 ms with 2, 1.156 ms with 4 (the row-to-row register moves of the prefetch and the
+// chords vanish; profiles/r3_tip_window_ab.json)
+#define AAI_WIN_ROW_UNROLL (AAI_MAXN - 1)
+#endif
+constexpr int kWinRowUnroll = AAI_WIN_ROW_UNROLL;
 // Columns that every interior footprint of this translation unit touches: a footprint box of side 2 ext holds at least
 // floor(2 ext) lattice columns, and the host picks the smallest MAXN >= floor(2 ext) + 1 (MAXN = 8 also serves
 // floor(2 ext) = 6, MAXN = 4 also floor(2 ext) = 2: L(c+s) < 2).  Their loads need no predicate; a pixel whose FP32 cell
@@ -199,10 +206,16 @@ enum { ADDR_GENERAL = 0, ADDR_IDENT = 1, ADDR_GROUPED = 2 };
 // honoured.  Measured (profiles/r2_z_pdl_ab.txt): the 8 bands of config 4 0.1844 -> 0.1824 ms, config 2 38 -> 36 us; the
 // two instructions cost ~80 ns per CTA on long launches, and even behind a run-time flag 0.7 % of the whole-canvas
 // launch -- hence a separate instantiation, used below kPdlMaxCtas CTAs only.
-template <typename TI, typename TO, int NC, int ADDR, bool STAGED, bool PDL = false, bool REV = false>
+// WIN (identity addressing, one channel, plans that pass aai_tip_window_ok): a fixed window of MAXN-1 rows x MAXN-1
+// columns from the footprint's first cell row and column, then the two tips of the footprint outside it in closed form
+// (aai_tip_strips_f32).  A box of D = L(c+s) < MAXN - 1 cells holds MAXN - 1 or MAXN cells per axis, but the
+// row loop runs to the warp's largest count and the columns are unrolled to MAXN, so every pixel paid for MAXN^2 cells.
+template <typename TI, typename TO, int NC, int ADDR, bool STAGED, bool PDL = false, bool REV = false, bool WIN = false>
 __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const char *stage, int spitch, int sox, int soy) {
     constexpr bool IDENT = ADDR == ADDR_IDENT, GROUPED = ADDR == ADDR_GROUPED;
     static_assert(!STAGED || IDENT, "staging is implemented for identity addressing");
+    static_assert(!WIN || (IDENT && NC == 1), "the cell window is implemented for identity addressing, one channel");
+    constexpr int NCOL = WIN ? MAXN - 1 : MAXN;  // cell columns evaluated per row
     if constexpr (PDL) asm volatile("griddepcontrol.launch_dependents;");
     // (no early return: every lane of a warp reaches the cooperative FP64 section at the end)
     const int x = blockIdx.x * TILE_W + threadIdx.x;
@@ -241,14 +254,15 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
     // Border pixels (footprint partly outside the image) are normalised by a partial, possibly tiny, total area:
     // they need relative accuracy, so they take the FP64 path (~0.1% of a large canvas).
     bool redo = work && (border || ncols > MAXN || nrows > MAXN || ncols < MINC);  // (the MAXN test cannot fire for the MAXN the host picked)
+    if (WIN) redo = redo || (work && nrows < MAXN - 1);  // the window's cells are read without predicates
     if (work && !redo) {
         const AaiShapeF &g = kp.shapef;
         const int dj0 = jy0 - iry;
         const float rx0 = (float)(ix0 - irx) - fx;
-        float yt[MAXN + 1], yb[MAXN + 1];
+        float yt[NCOL + 1], yb[NCOL + 1];
         if (!GROUPED) {
 #pragma unroll
-            for (int k = 0; k + 1 <= MAXN; k += 2) {  // two grid lines per packed instruction
+            for (int k = 0; k + 1 <= NCOL; k += 2) {  // two grid lines per packed instruction
                 AaiF2 t2, b2;
                 aai_chord_v_f32x2(g, aai_f2(rx0 + ((float)k - 0.5f), rx0 + ((float)k + 0.5f)), t2, b2);
                 yt[k] = t2.x;
@@ -256,7 +270,7 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
                 yb[k] = b2.x;
                 yb[k + 1] = b2.y;
             }
-            if ((MAXN + 1) & 1) aai_chord_v_f32(g, rx0 + ((float)MAXN - 0.5f), yt[MAXN], yb[MAXN]);
+            if ((NCOL + 1) & 1) aai_chord_v_f32(g, rx0 + ((float)NCOL - 0.5f), yt[NCOL], yb[NCOL]);
         }
         float xlT = 0.0f, xrT = 0.0f;  // chord of the footprint on the row's top grid line
         const float t0 = ((float)dj0 - fy) - 0.5f;  // top of row 0
@@ -307,23 +321,23 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
             aai_quadrant_areas_f32(g, e0 + (float)nA, t0 + (float)nT, nA < ncols, nT < nrows, W00, W01, W10, W11);
         }
         // lengths of the cells' top sides inside the footprint: the previous row's bottom sides
-        float lenTop[MAXN];
+        float lenTop[NCOL];
         if (!GROUPED) {
 #pragma unroll
-            for (int k = 0; k < MAXN; ++k) lenTop[k] = aai_overlap1_f32(xlT, xrT, e0 + (float)k);
+            for (int k = 0; k < NCOL; ++k) lenTop[k] = aai_overlap1_f32(xlT, xrT, e0 + (float)k);
         }
         // Source values are fetched one row ahead of their use (the loads of row r+1 are in flight while the areas of
         // row r are computed): the accumulate at the end of a row never waits for its own row's loads.
         // (Single-channel kernels only: three channels would need 30 staging registers.)
         constexpr bool PREFETCH = NC == 1 && !GROUPED;
-        float buf[MAXN][NC];
-        auto fetch = [&](int r, float (&v)[MAXN][NC]) {
+        float buf[NCOL][NC];
+        auto fetch = [&](int r, float (&v)[NCOL][NC]) {
             if (IDENT)
                 rowp = rowp0 + (int64_t)r * pitch;
             else
                 rowp = (const char *)kp.src + row_off(jy0 + r);
 #pragma unroll
-            for (int k = 0; k < MAXN; ++k) {
+            for (int k = 0; k < NCOL; ++k) {
 #pragma unroll
                 for (int ch = 0; ch < NC; ++ch) v[k][ch] = 0.0f;
                 if (k < MINC || k < ncols) {  // columns beyond the footprint box are never read (their area is exactly 0)
@@ -335,9 +349,10 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
         };
         if (PREFETCH) fetch(0, buf);
         // one row of cells: `cur` holds this row's source values (PREFETCH), `nxt` receives the next row's
-        auto row = [&](int r, float (&cur)[MAXN][NC], float (&nxt)[MAXN][NC]) {
+        const int nr = WIN ? MAXN - 1 : nrows;  // rows evaluated
+        auto row = [&](int r, float (&cur)[NCOL][NC], float (&nxt)[NCOL][NC]) {
             if (PREFETCH) {
-                if (r + 1 < nrows) fetch(r + 1, nxt);
+                if (r + 1 < nr) fetch(r + 1, nxt);
             } else {
                 rowp = IDENT ? rowp0 + (int64_t)r * pitch : (const char *)kp.src + row_off(jy0 + r);
             }
@@ -360,7 +375,7 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
             };
             // cells two at a time on the packed FP32 pipe (FFMA2/FMUL2/FADD2), a last odd cell on the scalar one
 #pragma unroll
-            for (int k = 0; k + 1 < MAXN; k += 2) {
+            for (int k = 0; k + 1 < NCOL; k += 2) {
                 const float rxa = rx0 + (float)k, rxb = rx0 + (float)(k + 1);
                 const float exa = rxa - 0.5f, exb = rxb - 0.5f;
                 // side lengths of the two cells: saturated ends on the scalar pipe, their differences packed
@@ -379,8 +394,8 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
                 take(k, area.x);
                 take(k + 1, area.y);
             }
-            if (MAXN & 1) {
-                constexpr int k = MAXN - 1;
+            if (NCOL & 1) {
+                constexpr int k = NCOL - 1;
                 const float rx = rx0 + (float)k;
                 const float ex = rx - 0.5f;
                 const float lenR = aai_overlap1_f32(yt[k + 1], yb[k + 1], ey);
@@ -392,17 +407,33 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
                 take(k, area);
             }
         };
-        if (!GROUPED) {
+        auto row_step = [&](int r) {
+            float nxt[NCOL][NC];
+            row(r, buf, nxt);
+            if (PREFETCH) {
+#pragma unroll
+                for (int k = 0; k < NCOL; ++k)
+#pragma unroll
+                    for (int ch = 0; ch < NC; ++ch) buf[k][ch] = nxt[k][ch];
+            }
+        };
+        if (WIN) {
+#pragma unroll kWinRowUnroll
+            for (int r = 0; r < MAXN - 1; ++r) row_step(r);
+        } else if (!GROUPED) {
 #pragma unroll kRowUnroll
-            for (int r = 0; r < nrows; ++r) {
-                float nxt[MAXN][NC];
-                row(r, buf, nxt);
-                if (PREFETCH) {
+            for (int r = 0; r < nrows; ++r) row_step(r);
+        }
+        if constexpr (WIN) {  // the right tip in column MAXN-1, the bottom tip in row MAXN-1
+            int first[2];
+            AaiF2 tip[3];
+            aai_tip_strips_f32<MAXN - 1>(g, e0, t0, first, tip);
+            // strips beyond the box have area 0: their loads are clamped into it
+            const char *colp = rowp0 + min(MAXN - 1, ncols - 1) * ESZ, *rowpb = rowp0 + min(MAXN - 1, nrows - 1) * pitch;
 #pragma unroll
-                    for (int k = 0; k < MAXN; ++k)
-#pragma unroll
-                        for (int ch = 0; ch < NC; ++ch) buf[k][ch] = nxt[k][ch];
-                }
+            for (int j = 0; j < 3; ++j) {
+                acc[0] = fmaf(LoadS<TI, STAGED>::get(colp + min(first[0] + j, nrows - 1) * pitch), tip[j].x, acc[0]);
+                acc[0] = fmaf(LoadS<TI, STAGED>::get(rowpb + min(first[1] + j, ncols - 1) * ESZ), tip[j].y, acc[0]);
             }
         }
         // Total overlap: the exact areas of a footprint inside the image add up to L^2 (border pixels never get here).
@@ -495,16 +526,16 @@ __device__ __forceinline__ void overlap_body(const AaiKernelParams &kp, const ch
     }
 }
 
-template <typename TI, typename TO, int NC, int ADDR, bool PDL = false, bool REV = false>
+template <typename TI, typename TO, int NC, int ADDR, bool PDL = false, bool REV = false, bool WIN = false>
 __global__ void __launch_bounds__(TILE_W *TILE_H, AAI_F32_MIN_BLOCKS)
     overlap_kernel_f32(const __grid_constant__ AaiKernelParams kp) {
-    overlap_body<TI, TO, NC, ADDR, false, PDL, REV>(kp, nullptr, 0, 0, 0);
+    overlap_body<TI, TO, NC, ADDR, false, PDL, REV, WIN>(kp, nullptr, 0, 0, 0);
 }
 #ifndef AAI_PDL
 #define AAI_PDL 1
 #endif
 constexpr long long kPdlMaxCtas = 150000;
-template <typename TI, typename TO, int NC>
+template <typename TI, typename TO, int NC, bool WIN>
 cudaError_t launch_short_pdl(const AaiKernelParams &kp, dim3 grid, dim3 block, cudaStream_t stream) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = grid;
@@ -516,12 +547,12 @@ cudaError_t launch_short_pdl(const AaiKernelParams &kp, dim3 grid, dim3 block, c
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (kp.reverse_rows) return cudaLaunchKernelEx(&cfg, overlap_kernel_f32<TI, TO, NC, ADDR_IDENT, true, true>, kp);
-    return cudaLaunchKernelEx(&cfg, overlap_kernel_f32<TI, TO, NC, ADDR_IDENT, true, false>, kp);
+    if (kp.reverse_rows) return cudaLaunchKernelEx(&cfg, overlap_kernel_f32<TI, TO, NC, ADDR_IDENT, true, true, WIN>, kp);
+    return cudaLaunchKernelEx(&cfg, overlap_kernel_f32<TI, TO, NC, ADDR_IDENT, true, false, WIN>, kp);
 }
 
 // the same kernel with the CTA's source window staged through shared memory by TMA (see "STAGED variants" above)
-template <typename TI, typename TO, int NC>
+template <typename TI, typename TO, int NC, bool WIN>
 __global__ void __launch_bounds__(TILE_W *TILE_H, AAI_F32_MIN_BLOCKS)
     overlap_kernel_f32_tma(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ AaiKernelParams kp,
                            const StageParams sp) {
@@ -530,21 +561,36 @@ __global__ void __launch_bounds__(TILE_W *TILE_H, AAI_F32_MIN_BLOCKS)
     __shared__ int origin[2];
     int sox, soy;
     stage_window<(int)sizeof(TI), NC>(&tmap, kp, sp, stage_raw, &bar, origin, kp.ext32, sox, soy);
-    overlap_body<TI, TO, NC, ADDR_IDENT, true>(kp, (const char *)stage_raw, sp.bw * (int)sizeof(TI), sox, soy);
+    overlap_body<TI, TO, NC, ADDR_IDENT, true, false, false, WIN>(kp, (const char *)stage_raw, sp.bw * (int)sizeof(TI), sox,
+                                                             soy);
 }
+
+// identity addressing: staged (A/B variant), short launches with PDL, or the whole-canvas kernel
+template <typename TI, typename TO, int NC, bool WIN>
+cudaError_t launch_ident(const AaiKernelParams &kp, dim3 grid, dim3 block, cudaStream_t stream) {
+    StageHost h;
+    if (kp.staged == 1 && stage_prepare<TI, NC>(kp, (double)kp.ext32, h)) {
+        overlap_kernel_f32_tma<TI, TO, NC, WIN><<<grid, block, h.smem, stream>>>(h.map, kp, h.sp);
+        return cudaGetLastError();
+    }
+    if (AAI_PDL && (long long)grid.x * grid.y * grid.z <= kPdlMaxCtas) return launch_short_pdl<TI, TO, NC, WIN>(kp, grid, block, stream);
+    overlap_kernel_f32<TI, TO, NC, ADDR_IDENT, false, false, WIN><<<grid, block, 0, stream>>>(kp);
+    return cudaGetLastError();
+}
+
+#ifndef AAI_TIP_WINDOW
+#define AAI_TIP_WINDOW 1  // 0: every plan takes the full MAXN x MAXN body (A/B builds)
+#endif
 
 template <typename TI, typename TO, int NC>
 cudaError_t launch3(const AaiKernelParams &kp, cudaStream_t stream) {
     if (kp.row1 <= kp.row0 || kp.dst_w <= 0) return cudaSuccess;
     const dim3 grid = canvas_grid(kp), block(TILE_W, TILE_H);
     if (kp.scale == 1 && kp.quadrant == 0) {
-        StageHost h;
-        if (kp.staged == 1 && stage_prepare<TI, NC>(kp, (double)kp.ext32, h)) {
-            overlap_kernel_f32_tma<TI, TO, NC><<<grid, block, h.smem, stream>>>(h.map, kp, h.sp);
-            return cudaGetLastError();
+        if constexpr (AAI_TIP_WINDOW && NC == 1) {
+            if (kp.tip_window) return launch_ident<TI, TO, NC, true>(kp, grid, block, stream);
         }
-        if (AAI_PDL && (long long)grid.x * grid.y * grid.z <= kPdlMaxCtas) return launch_short_pdl<TI, TO, NC>(kp, grid, block, stream);
-        overlap_kernel_f32<TI, TO, NC, ADDR_IDENT><<<grid, block, 0, stream>>>(kp);
+        return launch_ident<TI, TO, NC, false>(kp, grid, block, stream);
     } else if (MAXN == 4 && kp.scale >= MAXN - 1)
         overlap_kernel_f32<TI, TO, NC, (MAXN == 4 ? ADDR_GROUPED : ADDR_GENERAL)><<<grid, block, 0, stream>>>(kp);
     else
